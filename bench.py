@@ -5,6 +5,7 @@ calibrated exit threshold; exit-layer agreement %).
     python bench.py --gpus N --steps K --warmup W                     # headline: BASELINE.json configs[1]
     python bench.py --config sweep|large|image_only|fp32 ...          # the other BASELINE configs / the fp32 mode
     python bench.py --impl reference --gpus N --steps K ...           # the reference's CPU implementation (oracle port)
+    python bench.py ... --dump-outputs DIR                             # also write the last timed step's results as .npy
 
 A step = one pass of the hot path over one batch of synthetic RVL-CDIP-shaped documents
 (512 text tokens + boxes + 224x224 image, 16 classes).  Workloads (BASELINE.json `configs`):
@@ -52,6 +53,7 @@ SWEEP_THRESHOLDS = (0.5, 0.6, 0.7, 0.8, 0.9, 0.95, 0.99)
 SWEEP_DOCS = 8192
 AGREEMENT_DOCS = 16           # documents of the timed batch re-run through the oracle (exit_agreement)
 CPU_SAMPLE_DOCS = 16          # SURVEY.md §8(d): config 1 exactly (B = 16), 1 warm-up + 3 timed, median
+DUMP_LIMIT_BYTES = 64 << 20   # --dump-outputs: total size of the arrays written
 
 
 def workload(config: str):
@@ -191,6 +193,28 @@ def reached_per_layer(hist, exit_layers, n_layers, n_docs):
     return out
 
 
+def unpack_results(rows, K: int):
+    """Packed result rows [..., K + 2] (`mmee.dist.pack_results`) -> logits, exit index, criterion."""
+    return {"logits": rows[..., :K], "exit_index": rows[..., K].astype(np.int64), "criterion": rows[..., K + 1]}
+
+
+def dump_outputs(out_dir: str, arrays) -> None:
+    """`--dump-outputs`: write the results the timed path returned in its last step as `<out_dir>/<name>.npy` (floats
+    as they are, integer arrays as float64), so that two builds can be compared output for output on the same seeded
+    inputs.  The temperatures and thresholds come from the build's own calibration pass; they are written too, so
+    that a difference in exit indices can be told apart from a difference in calibration."""
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        out[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_port_time(dims, ee, sd, docs, threads: int) -> float:
     """One dense forward of the oracle port (reference algorithm, torch CPU fp32, every exit for every document)."""
     from oracle import port
@@ -303,7 +327,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-agreement", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step, gathered over the GPUs, and the calibrated "
+                         "temperatures and thresholds to DIR/<name>.npy (written by rank 0; the mmee path)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "mmee":
+        ap.error("--dump-outputs writes the results of the mmee path only")
     args.warmup = max(args.warmup, 3) if args.impl == "mmee" else args.warmup
 
     if args.impl == "reference":
@@ -447,6 +478,10 @@ def run_single(args, world, rank, local, dev):
     stage = model.last_stage_ms()          # per-stage CUDA-event times, averaged over the timed steps
     launches = model.last_launch_count()
     model.set_profiling(False)
+    if args.dump_outputs and rank == 0:    # the last step's rows of the job results: every rank's batch, in rank order
+        out = unpack_results(res["job_results"][(steps - 1) % cap].numpy(), K)
+        out["exit_hist"] = np.bincount(out["exit_index"], minlength=E1)
+        dump_outputs(args.dump_outputs, dict(out, temperatures=temps, thresholds=np.atleast_1d(thr)))
     value = world * B / (ms_step / 1000.0)
     clocks_all = [clk.summary()]
     if world > 1:
@@ -650,11 +685,13 @@ def run_sweep(args, world, rank, local, dev):
         model.infer_device(**shards[0], exit_threshold=thresholds_for(kind, 0.8, K), temperatures=temps)
     torch.cuda.synchronize()
     points = []
+    last_steps = []
     with ClockSampler(local, enabled=(rank == 0)) as clk:
         total_ms = 0.0
         for conf_thr in SWEEP_THRESHOLDS:
             ms, (host, hist) = timed_region(lambda: sweep_point(conf_thr), args.steps, 1, world, dev)
             total_ms += ms
+            last_steps.append((host, hist))
             reached = reached_per_layer(hist, model.exit_layers, dims.layers, n_total)
             flops = sum(reached) * (fl["linear"] + fl["attn"]) + n_total * fl["patch"]
             tf = flops / (ms / 1000.0) / 1e12
@@ -664,6 +701,11 @@ def run_sweep(args, world, rank, local, dev):
                            "predicted_classes_checksum": int(host[:, :K].argmax(1).sum())})
     launches = model.last_launch_count()
     value = n_total * len(SWEEP_THRESHOLDS) / (total_ms / 1000.0)
+    if args.dump_outputs and rank == 0:    # per threshold (axis 0): all documents of the job, gathered over the ranks
+        out = unpack_results(torch.stack([h for h, _ in last_steps]).numpy(), K)
+        out["exit_hist"] = np.stack([hs for _, hs in last_steps])
+        dump_outputs(args.dump_outputs, dict(out, temperatures=temps, thresholds=np.array(
+            [thresholds_for(kind, t, K) for t in SWEEP_THRESHOLDS])))
     if rank == 0:
         best = max(points, key=lambda p: p["algorithmic_tflops"])
         line = {

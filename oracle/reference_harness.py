@@ -73,14 +73,8 @@ def load():
     return L
 
 
-def build_reference_model(dims, ee, state_dict=None):
-    """Construct the reference `LayoutLMv3EEForSequenceClassification` for (dims, ee) in eval mode.
-
-    `ee.exits` must contain an embedding-level exit for encoder exits to be reported
-    (reference quirk, EE/models/LayoutLMv3.py:402,648-649)."""
-    import torch
-
-    L = load()
+def reference_config(dims, ee):
+    """The HF LayoutLMv3Config with the `EE_config` dict the reference model is constructed from."""
     cfg = dims.to_hf_config()
     cfg.EE_config = {
         "training_strategy": "one_stage_subgraphs_weighted",
@@ -93,6 +87,18 @@ def build_reference_model(dims, ee, state_dict=None):
     }
     if getattr(ee, "use_lte", False):
         cfg.EE_config["use_lte"] = True
+    return cfg
+
+
+def build_reference_model(dims, ee, state_dict=None):
+    """Construct the reference `LayoutLMv3EEForSequenceClassification` for (dims, ee) in eval mode.
+
+    `ee.exits` must contain an embedding-level exit for encoder exits to be reported
+    (reference quirk, EE/models/LayoutLMv3.py:402,648-649)."""
+    import torch
+
+    L = load()
+    cfg = reference_config(dims, ee)
     torch.manual_seed(0)
     model = L.LayoutLMv3EEForSequenceClassification(cfg).eval()
     if state_dict is not None:

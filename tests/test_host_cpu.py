@@ -201,9 +201,21 @@ def test_two_rank_gather_equals_single_process(tmp_path):
     assert all(open(os.path.join(tmp_path, f"ok{r}")).read() == "1" for r in range(world))
 
 
-@pytest.mark.skipif(not __import__("oracle.reference_harness", fromlist=["x"]).available(), reason="reference tree not present")
+class _ReferenceLike:
+    """What spec_from_reference reads off a reference model: its config (HF LayoutLMv3Config + EE_config, as the
+    reference is constructed) and the state dict it loaded strictly."""
+
+    def __init__(self, config, state_dict):
+        self.config = config
+        self._sd = state_dict
+
+    def state_dict(self):
+        return dict(self._sd)
+
+
 def test_spec_from_reference_model():
-    """from_reference() reads dims, exit config and weights off a constructed reference model."""
+    """from_reference() reads dims, exit config and weights off a constructed reference model (the reference itself
+    when its source tree is present, else an object with the same `.config` / `.state_dict()`)."""
     from mmee.model import B200EEForSequenceClassification
     from oracle import reference_harness as RH
 
@@ -211,7 +223,12 @@ def test_spec_from_reference_model():
     ee = ExitConfig.from_dict(dict(exits=["text_visual_concat", 1, 2], encoder_layer_strategy="gate",
                                    inference_strategy="entropy", global_threshold=0.4))
     sd = synth.make_state_dict(dims, ee, seed=1)
-    ref = RH.build_reference_model(dims, ee, sd)
+    if RH.available():
+        ref = RH.build_reference_model(dims, ee, sd)
+    else:
+        # checks the config half in full; the weight half only checks that names and values pass through, not that
+        # mmee.synth names parameters as the reference does (its strict load in build_reference_model checks that)
+        ref = _ReferenceLike(RH.reference_config(dims, ee), sd)
     d2, e2, sd2 = B200EEForSequenceClassification.spec_from_reference(ref)
     assert d2 == dims
     assert list(e2.exits) == list(ee.exits) and e2.encoder_layer_strategy == "gate" and e2.inference_strategy == "entropy"

@@ -1,6 +1,6 @@
 """CPU tests: the oracle port and policy port against the golden vectors (outputs of the
-unmodified reference, tests/golden/make_golden.py) and, when /root/reference is present,
-against the reference's own classes live."""
+unmodified reference, tests/golden/make_golden.py) and, when the original project's source tree is present
+(MMEE_REFERENCE_ROOT), against the reference's own classes live."""
 import os
 
 import numpy as np
@@ -68,7 +68,8 @@ def test_policy_edge_cases():
     assert (ex == 0).all()
 
 
-@pytest.mark.skipif(not reference_harness.available(), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not reference_harness.available(),
+                    reason="needs the original project's source tree (MMEE_REFERENCE_ROOT), which the repository does not contain")
 def test_port_matches_live_reference_tiny():
     from mmee import synth
     from mmee.config import ExitConfig, ModelDims
