@@ -123,7 +123,29 @@ int  mmee_forward_submit(mmee_engine* e, int B, const int64_t* input_ids, const 
                          const int64_t* attention_mask, const float* pixel_values, const mmee_policy* policy);
 int  mmee_forward_collect(mmee_engine* e, int ticket, const mmee_outputs* out);
 
-/* Number of kernels launched by the engine in the last forward (for the bench's gpu_launches). */
+/* Forward plans: one forward captured into a CUDA graph and instantiated, for a fixed batch size, criterion, mode and
+ * set of outputs.  A run launches the graph once instead of ~100 kernels, which is what a caller with few documents
+ * per call (the reference's eval loop runs one, EE/utils.py:169-193) pays for.  In early-exit mode every exit opens an
+ * IF node around the rest of the forward: once every document has left, the deeper layers are not launched at all.
+ * Thresholds and temperatures are inputs of every run (uploaded to the device before the graph starts), so one plan
+ * serves every policy.  A plan uses the engine's scratch buffers and staged-input buffers: its runs are ordered with
+ * the engine's other forwards, on any stream, as those are with each other.  Stage profiling (mmee_set_profiling)
+ * does not apply to plan runs. */
+typedef struct mmee_plan mmee_plan;
+/* Capture one forward for a fixed batch B <= max_batch.  criterion and mode come from `shape` (thresholds and
+ * temperatures are ignored here: they are inputs of every run); want_all = 1 also produces the all_* outputs.
+ * Creation runs one eager forward of neutral inputs first (kernel attributes, module loading) and synchronises. */
+int  mmee_plan_create(mmee_engine* e, int B, const mmee_policy* shape, int want_all, mmee_plan** out);
+/* Same inputs / outputs / errors as mmee_forward and mmee_forward_device, for exactly B documents; policy->criterion and
+ * policy->mode must equal the plan's.  Bit-identical results to the eager entry points. */
+int  mmee_plan_forward(mmee_plan* p, const int64_t* input_ids, const int64_t* bbox, const int64_t* attention_mask,
+                       const float* pixel_values, const mmee_policy* policy, const mmee_outputs* out);
+int  mmee_plan_forward_device(mmee_plan* p, const int64_t* input_ids, const int64_t* bbox, const int64_t* attention_mask,
+                              const float* pixel_values, const mmee_policy* policy, const mmee_outputs* out,
+                              void* cuda_stream);
+void mmee_plan_destroy(mmee_plan* p);   /* before mmee_destroy; mmee_destroy frees plans still alive */
+
+/* Number of kernels launched by the engine in the last eager forward (for the bench's gpu_launches). */
 int64_t mmee_last_launch_count(mmee_engine* e);
 /* Device time per stage ("total", "embed", "gemm", "attention", "norm", "exit"), SUMMED in ms over the forwards run
  * since profiling was switched on or last collected, and the number of those forwards ("forwards"): only recorded when
@@ -137,7 +159,8 @@ int  mmee_sync(mmee_engine* e, void* cuda_stream);
 int  mmee_collect_profile(mmee_engine* e);
 double mmee_last_stage_ms(mmee_engine* e, const char* stage);
 /* Test hook: copy an internal activation buffer ("X0","X1","QK","VT","CTX","A1","MID","Y","VIS","POOL","BIAS")
- * to host memory (synchronises the device). Returns bytes copied or < 0. */
+ * to host memory (synchronises the device). Returns bytes copied or < 0.  "NDEV": the active documents per exit stage
+ * (int32 [n_exits + 3]; a plan run first sets entries 1.. to -1, so a stage whose exit kernel was skipped reads -1). */
 int64_t mmee_debug_read(mmee_engine* e, const char* name, void* host_dst, int64_t capacity_bytes);
 
 /* Post-hoc exit policy over stored per-exit logits: the device replacement of the per-sample double loop of

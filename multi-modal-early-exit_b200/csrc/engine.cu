@@ -230,6 +230,9 @@ struct mmee_engine {
   } slots[2];
   int next_slot = 0;
   cudaEvent_t px_wait = nullptr;            // event forward_device waits on before touching pixels (px_async)
+  // captured forwards (mmee_plan_create): run on the same scratch buffers, freed by mmee_destroy if still alive
+  std::vector<mmee_plan*> plans;
+  bool capturing = false;                   // forward_device is recording a plan: no stage events
 
   ~mmee_engine() {
     for (auto& sl : slots) {
@@ -422,7 +425,7 @@ void launch_ln(mmee_engine* e, const float* Y, __nv_bfloat16* X, __nv_bfloat16* 
 }
 
 void mark(mmee_engine* e, const char* name, cudaStream_t st) {
-  if (!e->profiling) return;
+  if (!e->profiling || e->capturing) return;
   cudaEvent_t evn;
   CUDA_OK(cudaEventCreate(&evn));
   CUDA_OK(cudaEventRecord(evn, st));
@@ -708,8 +711,79 @@ void allocate(mmee_engine* e) {
 }
 
 // ------------------------------------------------------------------------------------------------ forward
+// Effective threshold and 1/T of exit x (x = n_exits: the final classifier) under `pol`: what exit_fused_kernel
+// compares against, as launch arguments (eager forwards) or uploaded before every run of a plan.
+void exit_policy(const mmee_engine* e, const mmee_policy* pol, int x, float* threshold, float* inv_temp) {
+  const mmee_model_desc& d = e->d;
+  const bool is_final = x == d.n_exits;
+  const float Te = pol->temperatures ? pol->temperatures[x] : 1.f;
+  *inv_temp = 1.0f / Te;
+  *threshold = is_final ? 0.f : pol->thresholds[x];
+  if (pol->criterion == MMEE_CRIT_LTE && !is_final) {
+    // the reference raises EarlyExitException only inside the encoder, at layer i + 1 < num_layers where
+    // num_layers = len(exit_encoder_layers) (EE/models/LayoutLMv3.py:139, 250-268); other exits are scored, never taken
+    int n_enc = 0;
+    for (int j = 0; j < d.n_exits; ++j) n_enc += d.exit_after_layer[j] > 0 ? 1 : 0;
+    const int code = d.exit_after_layer[x];
+    if (!(code > 0 && code < n_enc)) *threshold = -INFINITY;
+  }
+}
+
+// Capturing mode of forward_device (mmee_plan_create): the same launch sequence is recorded into a CUDA graph.  In
+// early-exit mode everything after an exit is captured into the body of an IF node whose condition the exit kernel
+// sets to "someone survived", so the IF nodes nest one per exit and the deeper layers are not launched at all once
+// every document has left.
+struct Capture {
+  const float* policy_dev = nullptr;   // [2 (E+1)] {threshold, 1/T} per exit, uploaded before every run
+  bool skip_tail = false;              // early-exit mode
+  cudaStream_t root = nullptr;         // captures the plan's graph
+  cudaStream_t side[2] = {};           // capture the body of the innermost IF node (alternating)
+  int depth = 0;                       // IF nodes opened so far
+};
+
+cudaGraph_t capturing_graph(cudaStream_t st, const cudaGraphNode_t** deps = nullptr, size_t* n_deps = nullptr) {
+  cudaStreamCaptureStatus status;
+  cudaGraph_t g = nullptr;
+  CUDA_OK(cudaStreamGetCaptureInfo(st, &status, nullptr, &g, deps, n_deps));
+  if (status != cudaStreamCaptureStatusActive) throw std::runtime_error("forward plan: stream capture is not active");
+  return g;
+}
+
+// condition of the next IF node, created in the graph being captured on `st` (where its node will be added)
+cudaGraphConditionalHandle capture_if_handle(cudaStream_t st) {
+  cudaGraphConditionalHandle h;
+  CUDA_OK(cudaGraphConditionalHandleCreate(&h, capturing_graph(st), 0, cudaGraphCondAssignDefault));
+  return h;
+}
+
+// adds an IF node on `h` after the work captured so far on `st` and returns the stream that captures its body
+cudaStream_t capture_open_if(Capture* cap, cudaStream_t st, cudaGraphConditionalHandle h) {
+  const cudaGraphNode_t* deps = nullptr;
+  size_t n_deps = 0;
+  cudaGraph_t g = capturing_graph(st, &deps, &n_deps);
+  cudaGraphNodeParams np{};
+  np.type = cudaGraphNodeTypeConditional;
+  np.conditional.handle = h;
+  np.conditional.type = cudaGraphCondTypeIf;
+  np.conditional.size = 1;
+  cudaGraphNode_t node;
+  CUDA_OK(cudaGraphAddNode(&node, g, deps, n_deps, &np));
+  // work captured on `st` from here on (the root stream only: the end of the forward) follows the IF node
+  CUDA_OK(cudaStreamUpdateCaptureDependencies(st, &node, 1, cudaStreamSetCaptureDependencies));
+  cudaStream_t body = cap->side[cap->depth & 1];
+  CUDA_OK(cudaStreamBeginCaptureToGraph(body, np.conditional.phGraph_out[0], nullptr, nullptr, 0,
+                                        cudaStreamCaptureModeThreadLocal));
+  if (st != cap->root) {                   // nothing else goes into an enclosing body
+    cudaGraph_t done = nullptr;
+    CUDA_OK(cudaStreamEndCapture(st, &done));
+  }
+  cap->depth += 1;
+  return body;
+}
+
 void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bbox, const int64_t* mask,
-                    const float* px, const mmee_policy* pol, const mmee_outputs* out, cudaStream_t st) {
+                    const float* px, const mmee_policy* pol, const mmee_outputs* out, cudaStream_t st,
+                    Capture* cap = nullptr) {
   if (!e->finalized) throw std::runtime_error("weights not finalized");
   if (B < 1 || B > e->max_batch) throw std::runtime_error("batch out of range");
   if (!pol || (e->d.n_exits > 0 && !pol->thresholds)) throw std::runtime_error("policy/thresholds missing");
@@ -723,14 +797,17 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
   const bool leave = pol->mode == 1;
   const bool gate = d.head_kind == 1;
   e->launches = 0;
-  if (!e->profiling || e->ev.size() > 100000) {          // profiling: the events of every forward since the last
-    for (auto& x : e->ev) cudaEventDestroy(x.second);    // collect are kept and folded together (stage averages)
+  if (!cap && (!e->profiling || e->ev.size() > 100000)) {  // profiling: the events of every forward since the last
+    for (auto& x : e->ev) cudaEventDestroy(x.second);      // collect are kept and folded together (stage averages)
     e->ev.clear();
   }
   // the engine has ONE set of scratch buffers: a forward on any stream is ordered after the previous forward (recorded
-  // at its end below), whichever stream that one ran on
-  CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
+  // at its end below), whichever stream that one ran on (a plan run does the same around its graph launch)
+  if (!cap) CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
   mark(e, "start", st);
+  if (cap) {   // stages whose exit kernel a run skips read -1 (mmee_debug_read "NDEV")
+    CUDA_OK(cudaMemsetAsync(e->n_dev.p + 1, 0xff, (e->n_dev.n - 1) * sizeof(int), st));
+  }
 
   init_forward_kernel<<<(std::max(B, E1) + 255) / 256, 256, 0, st>>>(e->slot_doc[0].p, e->out_exit.p, e->n_dev.p,
                                                                        e->m_dev.p, e->hist.p, B, S, E1);
@@ -780,19 +857,14 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     xa.gate_mode = use_cls ? 1 : 0;
     xa.n_labels = K;
     xa.criterion = pol->criterion;
-    const float Te = pol->temperatures ? pol->temperatures[exit_no] : 1.f;
-    xa.inv_temp = 1.0f / Te;
-    xa.threshold = is_final ? 0.f : pol->thresholds[exit_no];
+    exit_policy(e, pol, exit_no, &xa.threshold, &xa.inv_temp);
+    if (cap) xa.policy = cap->policy_dev + 2 * exit_no;
     xa.force = is_final ? 1 : 0;
     if (pol->criterion == MMEE_CRIT_LTE) {
-      // the reference raises EarlyExitException only inside the encoder, at layer i + 1 < num_layers where
-      // num_layers = len(exit_encoder_layers) (EE/models/LayoutLMv3.py:139, 250-268); other exits are scored, never taken
-      int n_enc = 0;
-      for (int x = 0; x < E; ++x) n_enc += d.exit_after_layer[x] > 0 ? 1 : 0;
-      const int code = is_final ? 0 : d.exit_after_layer[exit_no];
-      if (!is_final && !(code > 0 && code < n_enc)) xa.threshold = -INFINITY;
       xa.lte_w = e->lte_w.p; xa.lte_b = e->lte_b; xa.slot_lte = e->slot_lte.p;
     }
+    const bool open_if = cap && cap->skip_tail && !is_final;
+    if (open_if) { xa.cond = capture_if_handle(st); xa.set_cond = 1; }
     xa.slot_logits = e->slot_logits.p; xa.slot_head = e->slot_head.p; xa.slot_crit = e->slot_crit.p;
     xa.slot_fire = e->slot_fire.p;
     xa.group_ticket = e->exit_tickets.p; xa.groups_done = e->exit_tickets.p + (e->max_batch + EXF_DOCS - 1) / EXF_DOCS;
@@ -818,6 +890,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     exit_fused_kernel<<<grid, EXF_THREADS, smem, st>>>(xa);
     CUDA_OK(cudaGetLastError());
     e->launches++;
+    if (open_if) st = capture_open_if(cap, st, xa.cond);   // the rest of the forward runs only if someone survived
     stage += 1; sd ^= 1; rp ^= 1; exit_no += 1;
   };
 
@@ -1129,6 +1202,11 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
   }
 
   // ---- results (device -> caller's device buffers)
+  if (cap && st != cap->root) {            // close the innermost IF body: the rest follows the outermost IF node
+    cudaGraph_t done = nullptr;
+    CUDA_OK(cudaStreamEndCapture(st, &done));
+    st = cap->root;
+  }
   hist_to_i64_kernel<<<1, 64, 0, st>>>(e->hist.p, e->hist64.p, E1);
   e->launches++;
   auto d2d = [&](void* dst, const void* src, size_t bytes) {     // the host path hands in the engine's own buffers
@@ -1142,7 +1220,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
   d2d(out->all_criteria, e->all_crit.p, static_cast<size_t>(E1) * B * 4);
   d2d(out->exit_hist, e->hist64.p, static_cast<size_t>(E1) * 8);
   mark(e, "end", st);
-  CUDA_OK(cudaEventRecord(e->last_done, st));
+  if (!cap) CUDA_OK(cudaEventRecord(e->last_done, st));
 }
 
 // Device-side error flags, turned into errors by the synchronous entry points instead of returning garbage:
@@ -1179,6 +1257,154 @@ void collect_profile(mmee_engine* e) {
   e->stage_ms["forwards"] = forwards;
   for (auto& x : e->ev) cudaEventDestroy(x.second);
   e->ev.clear();
+}
+
+// staged inputs of the host paths and of plans, for max_batch documents
+void alloc_inputs(mmee_engine* e) {
+  if (e->in_ids.p) return;
+  const size_t mb = e->max_batch, T = e->T;
+  e->in_ids.alloc(mb * T); e->in_bbox.alloc(mb * T * 4); e->in_mask.alloc(mb * T);
+  e->in_px.alloc(mb * e->d.channels * e->d.image * e->d.image);
+}
+
+}  // namespace
+
+// A captured and instantiated forward for one (B, criterion, mode, want_all): include/mmee.h mmee_plan_create.
+struct mmee_plan {
+  mmee_engine* e = nullptr;
+  int B = 0, criterion = 0, mode = 0;
+  bool want_all = false;
+  DevBuf<float> policy_dev;                 // [2 (E+1)] {threshold, 1/T} per exit (exit_policy), read by the graph
+  float* policy_host = nullptr;             // pinned staging of policy_dev
+  cudaEvent_t policy_copied = nullptr;      // the previous run's upload of policy_host has completed
+  cudaGraph_t graph = nullptr;
+  cudaGraphExec_t exec = nullptr;
+  ~mmee_plan() {
+    if (exec) cudaGraphExecDestroy(exec);
+    if (graph) cudaGraphDestroy(graph);
+    if (policy_copied) cudaEventDestroy(policy_copied);
+    if (policy_host) cudaFreeHost(policy_host);
+  }
+};
+
+namespace {
+
+// One eager forward of B neutral documents (ids 0, boxes 0, mask 1, pixels 0): sets the kernel attributes (the
+// first-launch blocks of the launch helpers) and loads every module, neither of which may happen during a capture.
+void warm_up(mmee_engine* e, int B, int criterion) {
+  const size_t n_ids = static_cast<size_t>(B) * e->T, n_px = static_cast<size_t>(B) * e->d.channels * e->d.image * e->d.image;
+  cudaStream_t st = e->stream;
+  CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
+  std::vector<int64_t> ones(n_ids, 1);
+  CUDA_OK(cudaMemsetAsync(e->in_ids.p, 0, n_ids * 8, st));
+  CUDA_OK(cudaMemsetAsync(e->in_bbox.p, 0, n_ids * 32, st));
+  CUDA_OK(cudaMemcpyAsync(e->in_mask.p, ones.data(), n_ids * 8, cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaMemsetAsync(e->in_px.p, 0, n_px * 4, st));
+  std::vector<float> thr(std::max(e->d.n_exits, 1), 0.f);
+  const mmee_policy pol{criterion, 0, thr.data(), nullptr};
+  mmee_outputs dv{};                        // with the all_* outputs: every kernel a plan can contain is launched
+  dv.logits = e->out_logits.p; dv.exit_index = e->out_exit.p;
+  dv.all_exit_logits = e->all_logits.p; dv.all_head_logits = e->all_head.p; dv.all_criteria = e->all_crit.p;
+  forward_device(e, B, e->in_ids.p, e->in_bbox.p, e->in_mask.p, e->in_px.p, &pol, &dv, st);
+  CUDA_OK(cudaStreamSynchronize(st));
+  check_error_flags(e);
+}
+
+// Records forward_device for the plan into p->graph.  On failure every capture that was begun is ended and its graph
+// dropped, so the streams and the engine stay usable.
+void capture_plan(mmee_plan* p) {
+  mmee_engine* e = p->e;
+  Capture cap;
+  cap.policy_dev = p->policy_dev.p;
+  cap.skip_tail = p->mode == 1;
+  std::vector<float> thr(std::max(e->d.n_exits, 1), 0.f);   // ignored: the graph reads policy_dev
+  const mmee_policy pol{p->criterion, p->mode, thr.data(), nullptr};
+  mmee_outputs dv{};                        // results stay in the engine's own buffers
+  dv.logits = e->out_logits.p; dv.exit_index = e->out_exit.p; dv.criterion = e->out_crit.p;
+  dv.exit_hist = reinterpret_cast<int64_t*>(e->hist64.p);
+  if (p->want_all) { dv.all_exit_logits = e->all_logits.p; dv.all_head_logits = e->all_head.p; dv.all_criteria = e->all_crit.p; }
+  // ends a capture left open by a failure (a body graph belongs to its IF node, the root graph to nobody) and frees the
+  // stream
+  auto drop = [](cudaStream_t s, bool root) {
+    if (!s) return;
+    cudaStreamCaptureStatus status = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(s, &status) == cudaSuccess && status != cudaStreamCaptureStatusNone) {
+      cudaGraph_t g = nullptr;
+      cudaStreamEndCapture(s, &g);
+      if (g && root) cudaGraphDestroy(g);
+    }
+    cudaStreamDestroy(s);
+  };
+  try {
+    CUDA_OK(cudaStreamCreateWithFlags(&cap.root, cudaStreamNonBlocking));
+    CUDA_OK(cudaStreamCreateWithFlags(&cap.side[0], cudaStreamNonBlocking));
+    CUDA_OK(cudaStreamCreateWithFlags(&cap.side[1], cudaStreamNonBlocking));
+    CUDA_OK(cudaStreamBeginCapture(cap.root, cudaStreamCaptureModeThreadLocal));
+    e->capturing = true;
+    forward_device(e, p->B, e->in_ids.p, e->in_bbox.p, e->in_mask.p, e->in_px.p, &pol, &dv, cap.root, &cap);
+    e->capturing = false;
+    CUDA_OK(cudaStreamEndCapture(cap.root, &p->graph));
+  } catch (...) {
+    e->capturing = false;
+    drop(cap.side[0], false); drop(cap.side[1], false); drop(cap.root, true);
+    cudaGetLastError();
+    throw;
+  }
+  drop(cap.side[0], false); drop(cap.side[1], false); drop(cap.root, true);
+}
+
+// One run of a plan on `st`: inputs into the engine's staging buffers, the policy into policy_dev, the graph, results
+// out to the caller.  Ordered after the previous forward of the engine like every forward (last_done).
+void plan_run(mmee_plan* p, const int64_t* ids, const int64_t* bbox, const int64_t* mask, const float* px,
+              const mmee_policy* pol, const mmee_outputs* out, cudaStream_t st, bool host) {
+  mmee_engine* e = p->e;
+  const mmee_model_desc& d = e->d;
+  const int B = p->B, T = e->T, K = e->K, E = d.n_exits, E1 = E + 1;
+  if (!pol || (E > 0 && !pol->thresholds)) throw std::runtime_error("policy/thresholds missing");
+  if (pol->criterion != p->criterion || pol->mode != p->mode)
+    throw std::runtime_error("policy criterion / mode differ from the plan's (captured with criterion " +
+                             std::to_string(p->criterion) + ", mode " + std::to_string(p->mode) + ")");
+  if (!out || !out->logits || !out->exit_index) throw std::runtime_error("outputs missing");
+  if (!p->want_all && (out->all_exit_logits || out->all_head_logits || out->all_criteria))
+    throw std::runtime_error("all_* outputs need a plan created with want_all = 1");
+  if (!ids && T > 0) throw std::runtime_error("inputs missing");
+  if (!bbox && T > 0) throw std::runtime_error("inputs missing");
+  if (!mask && T > 0) throw std::runtime_error("inputs missing");
+  if (!px) throw std::runtime_error("inputs missing");
+  const size_t n_ids = static_cast<size_t>(B) * T, n_px = static_cast<size_t>(B) * d.channels * d.image * d.image;
+  const cudaMemcpyKind in_kind = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+  const cudaMemcpyKind out_kind = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  CUDA_OK(cudaEventSynchronize(p->policy_copied));           // the staging buffer is free again
+  for (int x = 0; x < E1; ++x) exit_policy(e, pol, x, &p->policy_host[2 * x], &p->policy_host[2 * x + 1]);
+  CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
+  if (n_ids) {
+    CUDA_OK(cudaMemcpyAsync(e->in_ids.p, ids, n_ids * 8, in_kind, st));
+    CUDA_OK(cudaMemcpyAsync(e->in_bbox.p, bbox, n_ids * 32, in_kind, st));
+    CUDA_OK(cudaMemcpyAsync(e->in_mask.p, mask, n_ids * 8, in_kind, st));
+  }
+  CUDA_OK(cudaMemcpyAsync(e->in_px.p, px, n_px * 4, in_kind, st));
+  CUDA_OK(cudaMemcpyAsync(p->policy_dev.p, p->policy_host, static_cast<size_t>(E1) * 2 * 4, cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaEventRecord(p->policy_copied, st));
+  CUDA_OK(cudaGraphLaunch(p->exec, st));
+  auto copy_out = [&](void* dst, const void* src, size_t bytes) {
+    if (dst) CUDA_OK(cudaMemcpyAsync(dst, src, bytes, out_kind, st));
+  };
+  copy_out(out->logits, e->out_logits.p, static_cast<size_t>(B) * K * 4);
+  copy_out(out->exit_index, e->out_exit.p, static_cast<size_t>(B) * 4);
+  copy_out(out->criterion, e->out_crit.p, static_cast<size_t>(B) * 4);
+  copy_out(out->all_exit_logits, e->all_logits.p, static_cast<size_t>(E1) * B * K * 4);
+  copy_out(out->all_head_logits, e->all_head.p, static_cast<size_t>(E1) * B * K * 4);
+  copy_out(out->all_criteria, e->all_crit.p, static_cast<size_t>(E1) * B * 4);
+  copy_out(out->exit_hist, e->hist64.p, static_cast<size_t>(E1) * 8);
+  CUDA_OK(cudaEventRecord(e->last_done, st));
+}
+
+void plan_destroy(mmee_plan* p) {
+  mmee_engine* e = p->e;
+  cudaSetDevice(e->device);
+  cudaEventSynchronize(e->last_done);       // the graph may still be running on a caller's stream
+  e->plans.erase(std::remove(e->plans.begin(), e->plans.end(), p), e->plans.end());
+  delete p;
 }
 
 }  // namespace
@@ -1269,6 +1495,7 @@ void mmee_destroy(mmee_engine* e) {
   if (!e) return;
   cudaSetDevice(e->device);
   cudaDeviceSynchronize();
+  while (!e->plans.empty()) plan_destroy(e->plans.back());
   delete e;
 }
 
@@ -1338,12 +1565,10 @@ int mmee_forward(mmee_engine* e, int B, const int64_t* input_ids, const int64_t*
   CUDA_OK(cudaSetDevice(e->device));
   const int T = e->T, K = e->K, E1 = e->d.n_exits + 1;
   const size_t n_ids = static_cast<size_t>(B) * T, n_px = static_cast<size_t>(B) * e->d.channels * e->d.image * e->d.image;
-  if (!e->in_ids.p) {
-    const size_t mb = e->max_batch;
-    e->in_ids.alloc(mb * T); e->in_bbox.alloc(mb * T * 4); e->in_mask.alloc(mb * T);
-    e->in_px.alloc(mb * e->d.channels * e->d.image * e->d.image);
-  }
+  alloc_inputs(e);
   cudaStream_t st = e->stream;
+  // a plan run on another stream may still read the staged inputs
+  CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
   // small inputs first (one H2D copy engine serves both streams in issue order); the pixels (96 % of the bytes) go up
   // on a second stream and are first needed by im2col, after text embedding and bias build
   CUDA_OK(cudaMemcpyAsync(e->in_ids.p, input_ids, n_ids * 8, cudaMemcpyHostToDevice, st));
@@ -1454,6 +1679,68 @@ int mmee_forward_collect(mmee_engine* e, int ticket, const mmee_outputs* out) {
   MMEE_CATCH
 }
 
+int mmee_plan_create(mmee_engine* e, int B, const mmee_policy* shape, int want_all, mmee_plan** out) {
+  MMEE_TRY
+  if (!e || !shape || !out) throw std::runtime_error("null argument");
+  if (!e->finalized) throw std::runtime_error("weights not finalized");
+  if (B < 1 || B > e->max_batch) throw std::runtime_error("batch out of range");
+  if (shape->criterion < 0 || shape->criterion > 2) throw std::runtime_error("criterion must be 0, 1 or 2");
+  if (shape->mode != 0 && shape->mode != 1) throw std::runtime_error("mode must be 0 (dense) or 1 (early exit)");
+  if (shape->criterion == MMEE_CRIT_LTE && !e->lte_w.p)
+    throw std::runtime_error("criterion LTE needs the weights layoutlmv3.encoder.lte_classifier.{weight,bias}");
+  CUDA_OK(cudaSetDevice(e->device));
+  alloc_inputs(e);
+  std::unique_ptr<mmee_plan> p(new mmee_plan());
+  p->e = e; p->B = B; p->criterion = shape->criterion; p->mode = shape->mode; p->want_all = want_all != 0;
+  const int E1 = e->d.n_exits + 1;
+  p->policy_dev.alloc(static_cast<size_t>(2) * E1, true);
+  CUDA_OK(cudaMallocHost(&p->policy_host, static_cast<size_t>(2) * E1 * sizeof(float)));
+  CUDA_OK(cudaEventCreateWithFlags(&p->policy_copied, cudaEventDisableTiming));
+  warm_up(e, B, p->criterion);
+  capture_plan(p.get());
+  CUDA_OK(cudaGraphInstantiate(&p->exec, p->graph, 0));
+  CUDA_OK(cudaGraphUpload(p->exec, e->stream));
+  CUDA_OK(cudaStreamSynchronize(e->stream));
+  e->plans.push_back(p.get());
+  *out = p.release();
+  return 0;
+  MMEE_CATCH
+}
+
+int mmee_plan_forward(mmee_plan* p, const int64_t* input_ids, const int64_t* bbox, const int64_t* attention_mask,
+                      const float* pixel_values, const mmee_policy* policy, const mmee_outputs* out) {
+  MMEE_TRY
+  if (!p) throw std::runtime_error("null plan");
+  mmee_engine* e = p->e;
+  CUDA_OK(cudaSetDevice(e->device));
+  plan_run(p, input_ids, bbox, attention_mask, pixel_values, policy, out, e->stream, true);
+  CUDA_OK(cudaStreamSynchronize(e->stream));
+  check_error_flags(e);
+  return 0;
+  MMEE_CATCH
+}
+
+int mmee_plan_forward_device(mmee_plan* p, const int64_t* input_ids, const int64_t* bbox, const int64_t* attention_mask,
+                             const float* pixel_values, const mmee_policy* policy, const mmee_outputs* out,
+                             void* cuda_stream) {
+  MMEE_TRY
+  if (!p) throw std::runtime_error("null plan");
+  mmee_engine* e = p->e;
+  CUDA_OK(cudaSetDevice(e->device));
+  cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : e->stream;
+  plan_run(p, input_ids, bbox, attention_mask, pixel_values, policy, out, st, false);
+  if (!cuda_stream) {
+    CUDA_OK(cudaStreamSynchronize(st));
+    check_error_flags(e);
+  }
+  return 0;
+  MMEE_CATCH
+}
+
+void mmee_plan_destroy(mmee_plan* p) {
+  if (p) plan_destroy(p);
+}
+
 int64_t mmee_last_launch_count(mmee_engine* e) { return e ? e->launches : -1; }
 
 int mmee_sync(mmee_engine* e, void* cuda_stream) {
@@ -1503,6 +1790,7 @@ int64_t mmee_debug_read(mmee_engine* e, const char* name, void* host_dst, int64_
     else if (n == "QKlo") { src = e->QKlo.p; bytes = e->QKlo.n * 2; }
     else if (n == "CTXlo") { src = e->CTXlo.p; bytes = e->CTXlo.n * 2; }
     else if (n == "MIDlo") { src = e->MIDlo.p; bytes = e->MIDlo.n * 2; }
+    else if (n == "NDEV") { src = e->n_dev.p; bytes = e->n_dev.n * 4; }
     else throw std::runtime_error("unknown buffer " + n);
     if (static_cast<int64_t>(bytes) > capacity_bytes) bytes = static_cast<size_t>(capacity_bytes);
     CUDA_OK(cudaMemcpy(host_dst, src, bytes, cudaMemcpyDeviceToHost));

@@ -630,7 +630,13 @@ struct ExitFusedArgs {
   float lte_b;              // own input row (EE/models/LayoutLMv3.py:142-149, 231-237); the class logits are unchanged
   float* slot_lte;          // [maxB] scratch
   float inv_temp, threshold;
+  const float* policy;      // optional (captured forward plans): {threshold, 1/T} of this exit in device memory, read
+                            // instead of the two scalars above so that one graph serves every policy
   int force;
+  // optional (captured forward plans, early-exit mode): the compacting thread sets this IF-node condition to
+  // "someone survived", so the launches of the deeper layers are skipped once every document has left
+  cudaGraphConditionalHandle cond;
+  int set_cond;
   float* slot_logits; float* slot_head; float* slot_crit; int* slot_fire;
   // tickets (zero on entry, reset by the last arriver)
   unsigned int* group_ticket;   // [ceil(maxB/16)]
@@ -722,7 +728,10 @@ __global__ void __launch_bounds__(EXF_THREADS) exit_fused_kernel(ExitFusedArgs a
   const int g = blockIdx.y;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if (n == 0) {                                 // nobody left: still publish the (empty) survivor list
-    if (blockIdx.x == 0 && g == 0 && blockIdx.z == 0) compact_block(a.compact, s_warp, s_misc);
+    if (blockIdx.x == 0 && g == 0 && blockIdx.z == 0) {
+      compact_block(a.compact, s_warp, s_misc);
+      if (a.set_cond && threadIdx.x == 0) cudaGraphSetConditional(a.cond, 0u);
+    }
     return;
   }
   if (g >= n_groups) return;
@@ -854,6 +863,8 @@ __global__ void __launch_bounds__(EXF_THREADS) exit_fused_kernel(ExitFusedArgs a
 
   // ---- (3) out_proj inputs into shared memory (T rows were written by other SMs: bypass L1)
   const int K = a.n_labels;
+  const float inv_temp = a.policy ? a.policy[1] : a.inv_temp;
+  const float threshold = a.policy ? a.policy[0] : a.threshold;
   if (a.head_src == 0 || a.head_src == 1) {
     const float* Tsrc = a.T[a.head_src];
     for (int i = threadIdx.x; i < EXF_DOCS * H / 4; i += EXF_THREADS) {
@@ -882,7 +893,7 @@ __global__ void __launch_bounds__(EXF_THREADS) exit_fused_kernel(ExitFusedArgs a
     float raw = head_val;                 // class logit of lane k
     if (a.gate_mode) raw = warp_dots_to_lanes(a.cls.out_w, a.cls.out_b, sX + dd * H, H, K, lane);
     if (lane < K) a.slot_logits[static_cast<size_t>(slot) * K + lane] = raw;
-    const float z = raw * a.inv_temp;
+    const float z = raw * inv_temp;
     const float zmax = warp_max(lane < K ? z : -INFINITY);
     const float ex = (lane < K) ? expf(z - zmax) : 0.f;
     const float A = warp_sum(ex);
@@ -897,7 +908,7 @@ __global__ void __launch_bounds__(EXF_THREADS) exit_fused_kernel(ExitFusedArgs a
     }
     if (lane == 0) {
       a.slot_crit[slot] = crit;
-      const bool fire = a.force || (a.criterion == 0 ? (crit > a.threshold) : (crit < a.threshold));
+      const bool fire = a.force || (a.criterion == 0 ? (crit > threshold) : (crit < threshold));
       a.slot_fire[slot] = fire ? 1 : 0;
     }
   }
@@ -911,6 +922,7 @@ __global__ void __launch_bounds__(EXF_THREADS) exit_fused_kernel(ExitFusedArgs a
   if (threadIdx.x == 0) *a.groups_done = 0u;
   __threadfence();
   compact_block(a.compact, s_warp, s_misc);
+  if (a.set_cond && threadIdx.x == 0) cudaGraphSetConditional(a.cond, s_misc[1] > 0 ? 1u : 0u);   // s_misc[1]: survivors
 }
 
 }  // namespace mmee

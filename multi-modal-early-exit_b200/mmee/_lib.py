@@ -20,6 +20,7 @@ EXPORTED_SYMBOLS = [
     "mmee_version", "mmee_policy_scan", "mmee_forward_submit", "mmee_forward_collect",
     "mmee_temperature_fit", "mmee_calibration_stats", "mmee_sync",
     "mmee_policy_store_create", "mmee_policy_store_destroy", "mmee_policy_store_criteria", "mmee_policy_store_scan",
+    "mmee_plan_create", "mmee_plan_forward", "mmee_plan_forward_device", "mmee_plan_destroy",
 ]
 
 
@@ -85,6 +86,15 @@ def load() -> C.CDLL:
     lib.mmee_forward_submit.restype = C.c_int
     lib.mmee_forward_collect.argtypes = [C.c_void_p, C.c_int, C.POINTER(Outputs)]
     lib.mmee_forward_collect.restype = C.c_int
+    lib.mmee_plan_create.argtypes = [C.c_void_p, C.c_int, C.POINTER(Policy), C.c_int, C.POINTER(C.c_void_p)]
+    lib.mmee_plan_create.restype = C.c_int
+    plan_args = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Policy), C.POINTER(Outputs)]
+    lib.mmee_plan_forward.argtypes = plan_args
+    lib.mmee_plan_forward.restype = C.c_int
+    lib.mmee_plan_forward_device.argtypes = plan_args + [C.c_void_p]
+    lib.mmee_plan_forward_device.restype = C.c_int
+    lib.mmee_plan_destroy.argtypes = [C.c_void_p]
+    lib.mmee_plan_destroy.restype = None
     lib.mmee_last_launch_count.argtypes = [C.c_void_p]
     lib.mmee_last_launch_count.restype = C.c_int64
     lib.mmee_set_profiling.argtypes = [C.c_void_p, C.c_int]

@@ -17,6 +17,7 @@ Everything numeric happens in the CUDA engine; torch is used for tensor storage 
 from __future__ import annotations
 
 import ctypes as C
+import weakref
 from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple, Union
 
@@ -102,6 +103,7 @@ class B200EEForSequenceClassification:
         self.exit_layers = sorted(EMBEDDING_EXIT_CODES[x] for x in ee.exits if isinstance(x, str)) \
             + sorted(ee.encoder_exit_layers)
         self.n_exits = len(self.exit_layers)
+        self._plans = weakref.WeakSet()     # live ForwardPlans: closed before the engine they run on
         self._lib = _lib.load()
         d = _lib.ModelDesc()
         d.hidden, d.layers, d.heads, d.inter = dims.hidden, dims.layers, dims.heads, dims.inter
@@ -160,6 +162,8 @@ class B200EEForSequenceClassification:
         _lib.check(self._lib.mmee_finalize_weights(self._h))
 
     def close(self) -> None:
+        for p in list(getattr(self, "_plans", ())):
+            p.close()
         if getattr(self, "_h", None) and self._h.value:
             self._lib.mmee_destroy(self._h)
             self._h = C.c_void_p()
@@ -185,7 +189,9 @@ class B200EEForSequenceClassification:
     # ------------------------------------------------------------------ engine call
     def _run(self, input_ids, attention_mask, bbox, pixel_values, criterion: str, mode: int,
              thresholds: Sequence[float], temperatures: Optional[Sequence[float]], want_all: bool,
-             blocking: bool = True):
+             blocking: bool = True, plan: Optional["ForwardPlan"] = None):
+        """One forward through the engine; `plan` given: a run of that captured forward plan instead (same inputs,
+        same outputs)."""
         if pixel_values is None:
             raise ValueError("pixel_values are required (multimodal and image-only paths)")
         if input_ids is None:
@@ -232,8 +238,16 @@ class B200EEForSequenceClassification:
             if tmp.shape[0] != E1:
                 raise ValueError(f"temperatures must have {E1} entries (one per exit + final)")
             pol.temperatures = tmp.ctypes.data_as(C.POINTER(C.c_float))
-        args = (self._h, B, C.c_void_p(ids.data_ptr()), C.c_void_p(bb.data_ptr()), C.c_void_p(msk.data_ptr()),
+        args = (C.c_void_p(ids.data_ptr()), C.c_void_p(bb.data_ptr()), C.c_void_p(msk.data_ptr()),
                 C.c_void_p(px.data_ptr()), C.byref(pol), C.byref(out))
+        if plan is None:
+            args = (self._h, B) + args
+            fwd_device, fwd_host = self._lib.mmee_forward_device, self._lib.mmee_forward
+        else:
+            if B != plan.batch_size:
+                raise ValueError(f"this plan was captured for {plan.batch_size} documents, got {B}")
+            args = (plan._handle(),) + args
+            fwd_device, fwd_host = self._lib.mmee_plan_forward_device, self._lib.mmee_plan_forward
         if on_dev:
             if dev.index is not None and dev.index != self.device_index:
                 raise ValueError("inputs live on a different GPU than the engine")
@@ -241,11 +255,11 @@ class B200EEForSequenceClassification:
             # synchronous": pass cudaStreamLegacy (1) instead, so the forward is ordered after the torch work that
             # produced the inputs and stays asynchronous; blocking callers wait explicitly below
             stream = torch.cuda.current_stream(dev).cuda_stream or 1
-            _lib.check(self._lib.mmee_forward_device(*args, C.c_void_p(stream)))
+            _lib.check(fwd_device(*args, C.c_void_p(stream)))
             if blocking:
                 _lib.check(self._lib.mmee_sync(self._h, C.c_void_p(stream)))
         else:
-            _lib.check(self._lib.mmee_forward(*args))
+            _lib.check(fwd_host(*args))
         return dict(logits=logits, exit_index=exit_index, criterion=crit, hist=hist, all_logits=all_l,
                     all_head=all_h, all_crit=all_c, _keep=(ids, msk, bb, px, thr, tmp))
 
@@ -285,6 +299,9 @@ class B200EEForSequenceClassification:
         crit_name = criterion or self._default_criterion()
         r = self._run(input_ids, attention_mask, bbox, pixel_values, crit_name, 1 if early_exit else 0,
                       np.atleast_1d(np.asarray(thr, dtype=np.float32)), temperatures, return_all)
+        return self._early_exit_result(r, return_all)
+
+    def _early_exit_result(self, r, return_all: bool) -> EarlyExitResult:
         ex = r["exit_index"].cpu().numpy().astype(np.int32)
         hist = r["hist"].cpu().numpy()
         n = ex.shape[0]
@@ -308,7 +325,23 @@ class B200EEForSequenceClassification:
         crit_name = criterion or self._default_criterion()
         r = self._run(input_ids, attention_mask, bbox, pixel_values, crit_name, 1 if early_exit else 0,
                       np.atleast_1d(np.asarray(thr, dtype=np.float32)), temperatures, False, blocking=False)
+        return self._device_result(r)
+
+    @staticmethod
+    def _device_result(r) -> Dict[str, torch.Tensor]:
         return {"logits": r["logits"], "exit_index": r["exit_index"], "criterion": r["criterion"], "hist": r["hist"]}
+
+    # ------------------------------------------------------------------ captured forwards
+    def plan(self, batch_size: int, criterion: Optional[str] = None, early_exit: bool = True,
+             return_all: bool = False) -> "ForwardPlan":
+        """Capture the forward for exactly `batch_size` documents into a CUDA graph (`mmee_plan_create`) and return
+        a `ForwardPlan` whose `infer` / `infer_device` run it: one graph launch per call instead of ~100 kernel
+        launches, and in early-exit mode no launches at all for the layers after the last document has left.
+        Thresholds and temperatures stay arguments of every call; the criterion, the mode and `return_all` are fixed
+        here.  Results are bit-identical to `infer` / `infer_device` on the same documents."""
+        p = ForwardPlan(self, batch_size, criterion or self._default_criterion(), early_exit, return_all)
+        self._plans.add(p)
+        return p
 
     # ------------------------------------------------------------------ pipelined host path
     def infer_submit(self, input_ids=None, attention_mask=None, bbox=None, pixel_values=None, labels=None,
@@ -404,6 +437,68 @@ class B200EEForSequenceClassification:
         buf = np.zeros(4096, dtype=np.uint8)
         n = self._lib.mmee_get_bucket_lut(self._h, which, buf.ctypes.data_as(C.c_void_p), buf.size)
         return buf[:n]
+
+
+class ForwardPlan:
+    """A forward captured for a fixed batch size, criterion, mode and `return_all` (`B200EEForSequenceClassification.plan`).
+
+    `infer` / `infer_device` take the same inputs as the model's methods of that name (host or CUDA tensors, same
+    rules) for exactly `batch_size` documents and return the same results, bit for bit.  The plan holds a reference to
+    its model; `close()` (or garbage collection) frees the graph."""
+
+    def __init__(self, model: B200EEForSequenceClassification, batch_size: int, criterion: str, early_exit: bool,
+                 return_all: bool):
+        if criterion not in CRITERION_CODES:
+            raise ValueError(f"criterion must be one of {sorted(CRITERION_CODES)}")
+        self.model = model
+        self.batch_size = int(batch_size)
+        self.criterion, self.early_exit, self.return_all = criterion, bool(early_exit), bool(return_all)
+        self._h = C.c_void_p()
+        shape = _lib.Policy()
+        shape.criterion = CRITERION_CODES[criterion]
+        shape.mode = 1 if early_exit else 0
+        _lib.check(model._lib.mmee_plan_create(model._h, self.batch_size, C.byref(shape), 1 if return_all else 0,
+                                               C.byref(self._h)))
+
+    def _handle(self) -> C.c_void_p:
+        if not self._h.value:
+            raise RuntimeError("this forward plan has been closed")
+        return self._h
+
+    def _call(self, batch, exit_threshold, temperatures, criterion, early_exit, want_all, blocking):
+        m = self.model
+        thr = m.ee.global_threshold if exit_threshold is None else exit_threshold
+        # criterion / early_exit default to the plan's; others are passed on and rejected by mmee_plan_forward
+        crit_name = criterion or self.criterion
+        mode = 1 if (self.early_exit if early_exit is None else early_exit) else 0
+        return m._run(batch.get("input_ids"), batch.get("attention_mask"), batch.get("bbox"),
+                      batch.get("pixel_values"), crit_name, mode, np.atleast_1d(np.asarray(thr, dtype=np.float32)),
+                      temperatures, want_all, blocking=blocking, plan=self)
+
+    def infer(self, exit_threshold: Union[float, Sequence[float], None] = None,
+              temperatures: Optional[Sequence[float]] = None, criterion: Optional[str] = None,
+              early_exit: Optional[bool] = None, **batch) -> EarlyExitResult:
+        """Same as `B200EEForSequenceClassification.infer` (with this plan's `return_all`)."""
+        r = self._call(batch, exit_threshold, temperatures, criterion, early_exit, self.return_all, True)
+        return self.model._early_exit_result(r, self.return_all)
+
+    def infer_device(self, exit_threshold: Union[float, Sequence[float], None] = None,
+                     temperatures: Optional[Sequence[float]] = None, criterion: Optional[str] = None,
+                     early_exit: Optional[bool] = None, **batch) -> Dict[str, torch.Tensor]:
+        """Same as `B200EEForSequenceClassification.infer_device`: asynchronous on the current stream."""
+        r = self._call(batch, exit_threshold, temperatures, criterion, early_exit, False, False)
+        return self.model._device_result(r)
+
+    def close(self) -> None:
+        if getattr(self, "_h", None) and self._h.value:
+            self.model._lib.mmee_plan_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def _entropy(x: torch.Tensor) -> torch.Tensor:
