@@ -411,8 +411,11 @@ void launch_ln(mmee_engine* e, const float* Y, __nv_bfloat16* X, __nv_bfloat16* 
   switch (H % 128 == 0 ? H / 128 : 0) {
     case 1: vec(std::integral_constant<int, 1>{}); break;
     case 2: vec(std::integral_constant<int, 2>{}); break;
+    case 3: vec(std::integral_constant<int, 3>{}); break;
     case 4: vec(std::integral_constant<int, 4>{}); break;
+    case 5: vec(std::integral_constant<int, 5>{}); break;
     case 6: vec(std::integral_constant<int, 6>{}); break;
+    case 7: vec(std::integral_constant<int, 7>{}); break;
     case 8: vec(std::integral_constant<int, 8>{}); break;
     default:
       if (stats_out) throw std::runtime_error("residual statistics need the vectorised LayerNorm (H % 128 == 0)");
@@ -918,8 +921,11 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
       switch (H / 128) {
         case 1: text_embed_vec_kernel<1><<<blocks, 256, 0, st>>>(ta, ew); break;
         case 2: text_embed_vec_kernel<2><<<blocks, 256, 0, st>>>(ta, ew); break;
+        case 3: text_embed_vec_kernel<3><<<blocks, 256, 0, st>>>(ta, ew); break;
         case 4: text_embed_vec_kernel<4><<<blocks, 256, 0, st>>>(ta, ew); break;
+        case 5: text_embed_vec_kernel<5><<<blocks, 256, 0, st>>>(ta, ew); break;
         case 6: text_embed_vec_kernel<6><<<blocks, 256, 0, st>>>(ta, ew); break;
+        case 7: text_embed_vec_kernel<7><<<blocks, 256, 0, st>>>(ta, ew); break;
         case 8: text_embed_vec_kernel<8><<<blocks, 256, 0, st>>>(ta, ew); break;
         default: scalar();
       }
@@ -975,8 +981,11 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     switch (H % 128 == 0 ? H / 128 : 0) {
       case 1: visual_ln_vec_kernel<1><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
       case 2: visual_ln_vec_kernel<2><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
+      case 3: visual_ln_vec_kernel<3><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
       case 4: visual_ln_vec_kernel<4><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
+      case 5: visual_ln_vec_kernel<5><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
       case 6: visual_ln_vec_kernel<6><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
+      case 7: visual_ln_vec_kernel<7><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
       case 8: visual_ln_vec_kernel<8><<<blocks, 256, 0, st>>>(e->VIS.p, ew, xo, wp, B, e->n_vis, T, S, H, d.vis_ln_eps, d.ln_eps); break;
       default:
         launch_nv(H, [&](auto nv) {
@@ -993,8 +1002,11 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     switch (H / 128) {
       case 1: embed_finish_vec_kernel<1><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
       case 2: embed_finish_vec_kernel<2><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
+      case 3: embed_finish_vec_kernel<3><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
       case 4: embed_finish_vec_kernel<4><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
+      case 5: embed_finish_vec_kernel<5><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
       case 6: embed_finish_vec_kernel<6><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
+      case 7: embed_finish_vec_kernel<7><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
       case 8: embed_finish_vec_kernel<8><<<blocks, 256, 0, st>>>(src, rows, map, ew, xout(cur), off, S, H, d.ln_eps, n_act); break;
       default: throw std::runtime_error("embedding-level exits need hidden % 128 == 0 and hidden <= 1024");
     }

@@ -421,22 +421,40 @@ def test_forwards_on_different_streams_are_ordered():
         assert torch.equal(r3.logits, ref.logits.cpu())
 
 
-@pytest.mark.parametrize("n_text,layers", [(77, 2), (200, 1), (448, 1)])
-def test_odd_sequence_lengths_vs_port(n_text, layers):
-    """Sequence lengths that are not 709: partial key / query tiles, other pitches.  Engine vs the oracle port."""
+# hidden size -> (coord, shape): 4 coord + 2 shape = hidden, both multiples of 4 so the vectorised text embedding runs
+HIDDEN_SPATIAL = {256: (40, 48), 384: (64, 64), 512: (88, 80), 640: (108, 104), 896: (152, 144)}
+
+
+@pytest.mark.parametrize("n_text,layers,hidden,dtype", [
+    pytest.param(77, 2, None, "bf16", id="77-2"), pytest.param(200, 1, None, "bf16", id="200-1"),
+    pytest.param(448, 1, None, "bf16", id="448-1")] + [
+    pytest.param(77, 1, h, dt, id=f"h{h}-{dt}") for h in sorted(HIDDEN_SPATIAL) for dt in ("bf16", "fp32")])
+def test_odd_sequence_lengths_vs_port(n_text, layers, hidden, dtype):
+    """Sequence lengths that are not 709: partial key / query tiles, other pitches.  Engine vs the oracle port.
+    `hidden`: every hidden size mmee_create accepts that the tiny / base / large models do not use (hidden / 128 = 2..7,
+    heads = hidden / 64), with the embedding-level exits, in both engine modes."""
     from mmee.model import B200EEForSequenceClassification
     from oracle import port
 
-    dims = ModelDims.tiny(n_text=n_text, layers=layers)
-    ee = ExitConfig.from_dict(dict(exits=["text_visual_concat"] + list(range(1, layers + 1)), encoder_layer_strategy="ramp",
-                                   inference_strategy="max_confidence"))
+    if hidden is None:
+        dims = ModelDims.tiny(n_text=n_text, layers=layers)
+        exits = ["text_visual_concat"] + list(range(1, layers + 1))
+    else:
+        coord, shape = HIDDEN_SPATIAL[hidden]
+        dims = ModelDims.tiny(n_text=n_text, layers=layers, hidden=hidden, heads=hidden // 64, inter=2 * hidden,
+                              coord=coord, shape=shape)
+        exits = ["vision_avg", "text_avg", "text_visual_concat", 1]
+    ee = ExitConfig.from_dict(dict(exits=exits, encoder_layer_strategy="ramp", inference_strategy="max_confidence"))
     sd = synth.make_state_dict(dims, ee, seed=5)
-    docs = synth.make_docs(dims, 5, seed=41, pad=True)
-    model = B200EEForSequenceClassification(dims, ee, sd, device=0, max_batch=8)
+    docs = synth.make_docs(dims, 5 if hidden is None else 4, seed=41, pad=True)
+    model = B200EEForSequenceClassification(dims, ee, sd, device=0, max_batch=8, dtype=dtype)
     got = model.forward(**_cuda(docs)).exit_logits.cpu().numpy()
     want = port.forward(sd, dims, ee, docs)["exit_logits"].numpy()
     assert np.isfinite(got).all()
-    assert np.abs(got - want).max() <= LOGIT_TOL
+    err = np.abs(got - want).max()
+    if hidden is not None:
+        print(f"hidden {hidden} [{dtype}]: max|logits - port| = {err:.3e}")
+    assert err <= TOL[dtype]
     dense = model.infer(**_cuda(docs), exit_threshold=0.2, early_exit=False)
     early = model.infer(**_cuda(docs), exit_threshold=0.2)
     assert np.array_equal(dense.exits_store, early.exits_store) and torch.equal(dense.logits, early.logits)
