@@ -113,6 +113,29 @@ int  mmee_forward_device(mmee_engine* e, int B, const int64_t* input_ids, const 
                          const int64_t* attention_mask, const float* pixel_values, const mmee_policy* policy,
                          const mmee_outputs* out, void* cuda_stream);
 
+/* Document images as uint8 pages, for callers that would otherwise run the LayoutLMv3 image processor on the host:
+ * the engine resizes, rescales and normalises them on the device, bit for bit as that processor does (Pillow's
+ * Image.resize((image, image), BILINEAR) of Image.fromarray(page).convert("RGB"), then (r / 255 - 0.5) / 0.5 in fp32;
+ * oracle/image_port.py).  Decoding stays with the caller. */
+typedef struct {
+  const uint8_t* data;     /* all B images back to back, row-major HWC */
+  const int64_t* offsets;  /* [B] byte offset of image b in data        (HOST memory) */
+  const int32_t* sizes;    /* [B, 2] (height, width), each in [1, 16384] (HOST memory) */
+  int channels;            /* 1 (grayscale) or 3 (RGB), the whole batch */
+  int64_t total_bytes;     /* size of data: what the host path uploads, and the bound every image is checked against */
+} mmee_images;
+/* data and pixel_values in DEVICE memory; pixel_values f32 [B, 3, image, image]; async on cuda_stream
+   (NULL = engine stream, synchronised).  Composes with mmee_forward_device and mmee_plan_forward_device.
+   Rejected before any launch: channels other than 1 or 3, a size outside [1, 16384], an image whose bytes run past
+   total_bytes, B outside [1, max_batch], an engine whose channels are not 3. */
+int  mmee_preprocess_images(mmee_engine* e, int B, const mmee_images* images, float* pixel_values, void* cuda_stream);
+/* mmee_forward with images (and everything else) in HOST memory instead of pixel_values.  The image bytes go up and
+   are preprocessed on the engine's copy stream, overlapping the text embedding and the bias build as the pixel upload
+   of mmee_forward does. */
+int  mmee_forward_images(mmee_engine* e, int B, const int64_t* input_ids, const int64_t* bbox,
+                         const int64_t* attention_mask, const mmee_images* images, const mmee_policy* policy,
+                         const mmee_outputs* out);
+
 /* Pipelined form of mmee_forward for throughput callers (a dataset loop such as EE/utils.py:169-193): up to TWO
  * forwards in flight, so the upload of batch n+1 (160 MB of pixels at 256 documents) overlaps the computation of
  * batch n.  submit enqueues the host->device copies, the forward and the result staging and returns a ticket (0 or 1)

@@ -21,6 +21,7 @@
 #include "attention.cuh"
 #include "embed.cuh"
 #include "gemm.cuh"
+#include "image.cuh"
 #include "norm_exit.cuh"
 #include "policy.cuh"
 #include "calibrate.cuh"
@@ -230,6 +231,14 @@ struct mmee_engine {
   } slots[2];
   int next_slot = 0;
   cudaEvent_t px_wait = nullptr;            // event forward_device waits on before touching pixels (px_async)
+  // uint8 image preprocess (image.cuh), grow-only: packed batch of the host path, first-pass intermediate,
+  // coefficient tables, and the per-call descriptors (ImageDesc[max_batch] + ImageAxis[2 max_batch]) with their pinned
+  // staging.  img_done orders preprocess calls on any streams (they share this scratch).
+  DevBuf<uint8_t> img_bytes, img_tmp, img_meta;
+  DevBuf<int> img_kk;
+  DevBuf<int2> img_bounds;
+  uint8_t* img_meta_host = nullptr;
+  cudaEvent_t img_meta_copied = nullptr, img_done = nullptr;
   // captured forwards (mmee_plan_create): run on the same scratch buffers, freed by mmee_destroy if still alive
   std::vector<mmee_plan*> plans;
   bool capturing = false;                   // forward_device is recording a plan: no stage events
@@ -246,6 +255,9 @@ struct mmee_engine {
     if (px_ready) cudaEventDestroy(px_ready);
     if (last_done) cudaEventDestroy(last_done);
     if (fwd_start) cudaEventDestroy(fwd_start);
+    if (img_meta_copied) cudaEventDestroy(img_meta_copied);
+    if (img_done) cudaEventDestroy(img_done);
+    if (img_meta_host) cudaFreeHost(img_meta_host);
   }
 };
 
@@ -1279,6 +1291,138 @@ void alloc_inputs(mmee_engine* e) {
   e->in_px.alloc(mb * e->d.channels * e->d.image * e->d.image);
 }
 
+// uint8 images (mmee_images, image.cuh): every check runs on the host, before anything is enqueued
+void check_images(const mmee_engine* e, int B, const mmee_images* im) {
+  if (!im || !im->data || !im->offsets || !im->sizes) throw std::runtime_error("images: data, offsets and sizes are required");
+  if (e->d.channels != 3)
+    throw std::runtime_error("uint8 images need an engine with channels = 3, this one has " + std::to_string(e->d.channels));
+  if (B < 1 || B > e->max_batch) throw std::runtime_error("batch out of range");
+  if (im->channels != 1 && im->channels != 3)
+    throw std::runtime_error("images: channels must be 1 (grayscale) or 3 (RGB), got " + std::to_string(im->channels));
+  for (int b = 0; b < B; ++b) {
+    const int h = im->sizes[2 * b], w = im->sizes[2 * b + 1];
+    if (h < 1 || h > IMG_MAX_SIDE || w < 1 || w > IMG_MAX_SIDE)
+      throw std::runtime_error("image " + std::to_string(b) + ": size (" + std::to_string(h) + ", " + std::to_string(w) +
+                               ") outside [1, " + std::to_string(IMG_MAX_SIDE) + "]");
+    const int64_t off = im->offsets[b], n = static_cast<int64_t>(h) * w * im->channels;
+    if (off < 0 || off > im->total_bytes - n)
+      throw std::runtime_error("image " + std::to_string(b) + ": bytes [" + std::to_string(off) + ", " +
+                               std::to_string(off + n) + ") run past total_bytes = " + std::to_string(im->total_bytes));
+  }
+}
+
+// Enqueues the preprocess of a checked batch on `st`: packed bytes `data` (device) -> px f32 [B, 3, S, S] (device).
+// Coefficient tables are computed once per distinct input length; scratch grows, it is never allocated per call.
+void preprocess_images(mmee_engine* e, int B, const mmee_images* im, const uint8_t* data, float* px, cudaStream_t st) {
+  const int S = e->d.image, C = im->channels;
+  const size_t desc_bytes = sizeof(ImageDesc) * e->max_batch, meta_bytes = desc_bytes + sizeof(ImageAxis) * 2 * e->max_batch;
+  if (!e->img_meta_host) {
+    CUDA_OK(cudaMallocHost(&e->img_meta_host, meta_bytes));
+    e->img_meta.alloc(meta_bytes);
+    e->img_bounds.alloc(static_cast<size_t>(2) * e->max_batch * S);
+    CUDA_OK(cudaEventCreateWithFlags(&e->img_meta_copied, cudaEventDisableTiming));
+    CUDA_OK(cudaEventCreateWithFlags(&e->img_done, cudaEventDisableTiming));
+  }
+  std::vector<ImageDesc> desc(B);
+  std::vector<ImageAxis> axes;
+  std::map<int, int> table;                 // input length -> coefficient table
+  int64_t kk_n = 0, tmp_n = 0, max_items = 0;
+  auto axis = [&](int in) {
+    auto it = table.find(in);
+    if (it != table.end()) return it->second;
+    const int ksize = 2 * std::max(1, (in + S - 1) / S) + 1;   // Pillow: 2 ceil(max(in / S, 1)) + 1
+    axes.push_back(ImageAxis{in, ksize, kk_n});
+    kk_n += static_cast<int64_t>(S) * ksize;
+    return table[in] = static_cast<int>(axes.size()) - 1;
+  };
+  for (int b = 0; b < B; ++b) {
+    ImageDesc& dsc = desc[b];
+    dsc.h = im->sizes[2 * b]; dsc.w = im->sizes[2 * b + 1];
+    dsc.src_off = im->offsets[b];
+    dsc.th = axis(dsc.h); dsc.tw = axis(dsc.w);
+    // Pillow's Image.resize shrinks a page more than 100 times taller than wide vertically first
+    dsc.vfirst = dsc.h > 100 * dsc.w && S < dsc.h;
+    dsc.pad_ = 0;
+    const int64_t items = dsc.vfirst ? static_cast<int64_t>(S) * dsc.w : static_cast<int64_t>(dsc.h) * S;
+    dsc.tmp_off = tmp_n;
+    tmp_n += items * C;
+    max_items = std::max(max_items, items);
+  }
+  if (static_cast<int64_t>(e->img_kk.n) < kk_n || static_cast<int64_t>(e->img_tmp.n) < tmp_n) {
+    CUDA_OK(cudaEventSynchronize(e->img_done));             // a preprocess on another stream may still read them
+    if (static_cast<int64_t>(e->img_kk.n) < kk_n) e->img_kk.alloc(kk_n);
+    if (static_cast<int64_t>(e->img_tmp.n) < tmp_n) e->img_tmp.alloc(tmp_n);
+  }
+  CUDA_OK(cudaEventSynchronize(e->img_meta_copied));        // the staging buffer is free again
+  memcpy(e->img_meta_host, desc.data(), sizeof(ImageDesc) * B);
+  memcpy(e->img_meta_host + desc_bytes, axes.data(), sizeof(ImageAxis) * axes.size());
+  CUDA_OK(cudaStreamWaitEvent(st, e->img_done, 0));
+  CUDA_OK(cudaMemcpyAsync(e->img_meta.p, e->img_meta_host, meta_bytes, cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaEventRecord(e->img_meta_copied, st));
+  const auto* d_desc = reinterpret_cast<const ImageDesc*>(e->img_meta.p);
+  const auto* d_axes = reinterpret_cast<const ImageAxis*>(e->img_meta.p + desc_bytes);
+  image_coeffs_kernel<<<static_cast<unsigned>(axes.size()), 128, 0, st>>>(d_axes, S, e->img_bounds.p, e->img_kk.p);
+  const unsigned gy = static_cast<unsigned>(std::min(B, 65535));
+  const dim3 g1(static_cast<unsigned>(std::min<int64_t>((max_items + 255) / 256, 1024)), gy);
+  const dim3 g2(static_cast<unsigned>(std::min<int64_t>((static_cast<int64_t>(S) * S + 255) / 256, 1024)), gy);
+  if (C == 1) {
+    image_pass1_kernel<1><<<g1, 256, 0, st>>>(data, d_desc, B, S, d_axes, e->img_bounds.p, e->img_kk.p, e->img_tmp.p);
+    image_pass2_kernel<1><<<g2, 256, 0, st>>>(e->img_tmp.p, d_desc, B, S, d_axes, e->img_bounds.p, e->img_kk.p, px);
+  } else {
+    image_pass1_kernel<3><<<g1, 256, 0, st>>>(data, d_desc, B, S, d_axes, e->img_bounds.p, e->img_kk.p, e->img_tmp.p);
+    image_pass2_kernel<3><<<g2, 256, 0, st>>>(e->img_tmp.p, d_desc, B, S, d_axes, e->img_bounds.p, e->img_kk.p, px);
+  }
+  CUDA_OK(cudaGetLastError());
+  CUDA_OK(cudaEventRecord(e->img_done, st));
+}
+
+// mmee_forward / mmee_forward_images: inputs and outputs in host memory.  The small inputs go up on the engine's
+// stream; `stage_pixels(copy_stream)` enqueues what fills in_px (96 % of the bytes), which overlaps the text embedding
+// and bias build and is first needed by im2col.
+template <typename F>
+void host_forward(mmee_engine* e, int B, const int64_t* input_ids, const int64_t* bbox, const int64_t* attention_mask,
+                  const mmee_policy* policy, const mmee_outputs* out, F&& stage_pixels) {
+  const int T = e->T, K = e->K, E1 = e->d.n_exits + 1;
+  const size_t n_ids = static_cast<size_t>(B) * T;
+  alloc_inputs(e);
+  cudaStream_t st = e->stream;
+  // a plan run on another stream may still read the staged inputs
+  CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
+  // small inputs first (one H2D copy engine serves both streams in issue order)
+  CUDA_OK(cudaMemcpyAsync(e->in_ids.p, input_ids, n_ids * 8, cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaMemcpyAsync(e->in_bbox.p, bbox, n_ids * 32, cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaMemcpyAsync(e->in_mask.p, attention_mask, n_ids * 8, cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaEventRecord(e->fwd_start, st));
+  CUDA_OK(cudaStreamWaitEvent(e->copy_stream, e->fwd_start, 0));       // previous forward has released in_px
+  stage_pixels(e->copy_stream);
+  CUDA_OK(cudaEventRecord(e->px_ready, e->copy_stream));
+  e->px_async = true;
+  // run with outputs in the engine's own device buffers, then copy what was asked for to the host
+  mmee_outputs dv{};
+  dv.logits = e->out_logits.p; dv.exit_index = e->out_exit.p; dv.criterion = e->out_crit.p;
+  dv.exit_hist = reinterpret_cast<int64_t*>(e->hist64.p);
+  if (out->all_exit_logits) dv.all_exit_logits = e->all_logits.p;
+  if (out->all_head_logits) dv.all_head_logits = e->all_head.p;
+  if (out->all_criteria) dv.all_criteria = e->all_crit.p;
+  try {
+    forward_device(e, B, e->in_ids.p, e->in_bbox.p, e->in_mask.p, e->in_px.p, policy, &dv, st);
+  } catch (...) {
+    e->px_async = false;
+    throw;
+  }
+  e->px_async = false;
+  CUDA_OK(cudaMemcpyAsync(out->logits, dv.logits, static_cast<size_t>(B) * K * 4, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaMemcpyAsync(out->exit_index, dv.exit_index, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, st));
+  if (out->criterion) CUDA_OK(cudaMemcpyAsync(out->criterion, dv.criterion, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, st));
+  if (out->exit_hist) CUDA_OK(cudaMemcpyAsync(out->exit_hist, dv.exit_hist, static_cast<size_t>(E1) * 8, cudaMemcpyDeviceToHost, st));
+  if (out->all_exit_logits) CUDA_OK(cudaMemcpyAsync(out->all_exit_logits, dv.all_exit_logits, static_cast<size_t>(E1) * B * K * 4, cudaMemcpyDeviceToHost, st));
+  if (out->all_head_logits) CUDA_OK(cudaMemcpyAsync(out->all_head_logits, dv.all_head_logits, static_cast<size_t>(E1) * B * K * 4, cudaMemcpyDeviceToHost, st));
+  if (out->all_criteria) CUDA_OK(cudaMemcpyAsync(out->all_criteria, dv.all_criteria, static_cast<size_t>(E1) * B * 4, cudaMemcpyDeviceToHost, st));
+  CUDA_OK(cudaStreamSynchronize(st));
+  collect_profile(e);
+  check_error_flags(e);
+}
+
 }  // namespace
 
 // A captured and instantiated forward for one (B, criterion, mode, want_all): include/mmee.h mmee_plan_create.
@@ -1575,46 +1719,40 @@ int mmee_forward(mmee_engine* e, int B, const int64_t* input_ids, const int64_t*
   if (!e || !out) throw std::runtime_error("null argument");
   if (B < 1 || B > e->max_batch) throw std::runtime_error("batch out of range");
   CUDA_OK(cudaSetDevice(e->device));
-  const int T = e->T, K = e->K, E1 = e->d.n_exits + 1;
-  const size_t n_ids = static_cast<size_t>(B) * T, n_px = static_cast<size_t>(B) * e->d.channels * e->d.image * e->d.image;
-  alloc_inputs(e);
-  cudaStream_t st = e->stream;
-  // a plan run on another stream may still read the staged inputs
-  CUDA_OK(cudaStreamWaitEvent(st, e->last_done, 0));
-  // small inputs first (one H2D copy engine serves both streams in issue order); the pixels (96 % of the bytes) go up
-  // on a second stream and are first needed by im2col, after text embedding and bias build
-  CUDA_OK(cudaMemcpyAsync(e->in_ids.p, input_ids, n_ids * 8, cudaMemcpyHostToDevice, st));
-  CUDA_OK(cudaMemcpyAsync(e->in_bbox.p, bbox, n_ids * 32, cudaMemcpyHostToDevice, st));
-  CUDA_OK(cudaMemcpyAsync(e->in_mask.p, attention_mask, n_ids * 8, cudaMemcpyHostToDevice, st));
-  CUDA_OK(cudaEventRecord(e->fwd_start, st));
-  CUDA_OK(cudaStreamWaitEvent(e->copy_stream, e->fwd_start, 0));       // previous forward has released in_px
-  CUDA_OK(cudaMemcpyAsync(e->in_px.p, pixel_values, n_px * 4, cudaMemcpyHostToDevice, e->copy_stream));
-  CUDA_OK(cudaEventRecord(e->px_ready, e->copy_stream));
-  e->px_async = true;
-  // run with outputs in the engine's own device buffers, then copy what was asked for to the host
-  mmee_outputs dv{};
-  dv.logits = e->out_logits.p; dv.exit_index = e->out_exit.p; dv.criterion = e->out_crit.p;
-  dv.exit_hist = reinterpret_cast<int64_t*>(e->hist64.p);
-  if (out->all_exit_logits) dv.all_exit_logits = e->all_logits.p;
-  if (out->all_head_logits) dv.all_head_logits = e->all_head.p;
-  if (out->all_criteria) dv.all_criteria = e->all_crit.p;
-  try {
-    forward_device(e, B, e->in_ids.p, e->in_bbox.p, e->in_mask.p, e->in_px.p, policy, &dv, st);
-  } catch (...) {
-    e->px_async = false;
-    throw;
-  }
-  e->px_async = false;
-  CUDA_OK(cudaMemcpyAsync(out->logits, dv.logits, static_cast<size_t>(B) * K * 4, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaMemcpyAsync(out->exit_index, dv.exit_index, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, st));
-  if (out->criterion) CUDA_OK(cudaMemcpyAsync(out->criterion, dv.criterion, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, st));
-  if (out->exit_hist) CUDA_OK(cudaMemcpyAsync(out->exit_hist, dv.exit_hist, static_cast<size_t>(E1) * 8, cudaMemcpyDeviceToHost, st));
-  if (out->all_exit_logits) CUDA_OK(cudaMemcpyAsync(out->all_exit_logits, dv.all_exit_logits, static_cast<size_t>(E1) * B * K * 4, cudaMemcpyDeviceToHost, st));
-  if (out->all_head_logits) CUDA_OK(cudaMemcpyAsync(out->all_head_logits, dv.all_head_logits, static_cast<size_t>(E1) * B * K * 4, cudaMemcpyDeviceToHost, st));
-  if (out->all_criteria) CUDA_OK(cudaMemcpyAsync(out->all_criteria, dv.all_criteria, static_cast<size_t>(E1) * B * 4, cudaMemcpyDeviceToHost, st));
-  CUDA_OK(cudaStreamSynchronize(st));
-  collect_profile(e);
-  check_error_flags(e);
+  const size_t n_px = static_cast<size_t>(B) * e->d.channels * e->d.image * e->d.image;
+  host_forward(e, B, input_ids, bbox, attention_mask, policy, out, [&](cudaStream_t cs) {
+    CUDA_OK(cudaMemcpyAsync(e->in_px.p, pixel_values, n_px * 4, cudaMemcpyHostToDevice, cs));
+  });
+  return 0;
+  MMEE_CATCH
+}
+
+int mmee_forward_images(mmee_engine* e, int B, const int64_t* input_ids, const int64_t* bbox,
+                        const int64_t* attention_mask, const mmee_images* images, const mmee_policy* policy,
+                        const mmee_outputs* out) {
+  MMEE_TRY
+  if (!e || !out) throw std::runtime_error("null argument");
+  check_images(e, B, images);
+  CUDA_OK(cudaSetDevice(e->device));
+  // the previous host forward has finished (it synchronises), so nothing reads img_bytes any more
+  if (static_cast<int64_t>(e->img_bytes.n) < images->total_bytes) e->img_bytes.alloc(images->total_bytes);
+  host_forward(e, B, input_ids, bbox, attention_mask, policy, out, [&](cudaStream_t cs) {
+    CUDA_OK(cudaMemcpyAsync(e->img_bytes.p, images->data, images->total_bytes, cudaMemcpyHostToDevice, cs));
+    preprocess_images(e, B, images, e->img_bytes.p, e->in_px.p, cs);
+  });
+  return 0;
+  MMEE_CATCH
+}
+
+int mmee_preprocess_images(mmee_engine* e, int B, const mmee_images* images, float* pixel_values, void* cuda_stream) {
+  MMEE_TRY
+  if (!e) throw std::runtime_error("null engine");
+  check_images(e, B, images);
+  if (!pixel_values) throw std::runtime_error("pixel_values missing");
+  CUDA_OK(cudaSetDevice(e->device));
+  cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : e->stream;
+  preprocess_images(e, B, images, images->data, pixel_values, st);
+  if (!cuda_stream) CUDA_OK(cudaStreamSynchronize(st));
   return 0;
   MMEE_CATCH
 }

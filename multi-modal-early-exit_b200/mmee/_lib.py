@@ -21,6 +21,7 @@ EXPORTED_SYMBOLS = [
     "mmee_temperature_fit", "mmee_calibration_stats", "mmee_sync",
     "mmee_policy_store_create", "mmee_policy_store_destroy", "mmee_policy_store_criteria", "mmee_policy_store_scan",
     "mmee_plan_create", "mmee_plan_forward", "mmee_plan_forward_device", "mmee_plan_destroy",
+    "mmee_preprocess_images", "mmee_forward_images",
 ]
 
 
@@ -49,6 +50,13 @@ class Outputs(C.Structure):
         ("logits", C.c_void_p), ("exit_index", C.c_void_p), ("criterion", C.c_void_p),
         ("all_exit_logits", C.c_void_p), ("all_head_logits", C.c_void_p), ("all_criteria", C.c_void_p),
         ("exit_hist", C.c_void_p),
+    ]
+
+
+class Images(C.Structure):
+    _fields_ = [
+        ("data", C.c_void_p), ("offsets", C.c_void_p), ("sizes", C.c_void_p), ("channels", C.c_int),
+        ("total_bytes", C.c_int64),
     ]
 
 
@@ -82,6 +90,11 @@ def load() -> C.CDLL:
     lib.mmee_forward.restype = C.c_int
     lib.mmee_forward_device.argtypes = fwd_args + [C.c_void_p]
     lib.mmee_forward_device.restype = C.c_int
+    lib.mmee_forward_images.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Images),
+                                         C.POINTER(Policy), C.POINTER(Outputs)]
+    lib.mmee_forward_images.restype = C.c_int
+    lib.mmee_preprocess_images.argtypes = [C.c_void_p, C.c_int, C.POINTER(Images), C.c_void_p, C.c_void_p]
+    lib.mmee_preprocess_images.restype = C.c_int
     lib.mmee_forward_submit.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Policy)]
     lib.mmee_forward_submit.restype = C.c_int
     lib.mmee_forward_collect.argtypes = [C.c_void_p, C.c_int, C.POINTER(Outputs)]

@@ -26,6 +26,7 @@ import torch
 
 from . import _lib
 from .config import ExitConfig, ModelDims
+from .images import PackedImages, as_packed
 
 
 @dataclass
@@ -189,29 +190,46 @@ class B200EEForSequenceClassification:
     # ------------------------------------------------------------------ engine call
     def _run(self, input_ids, attention_mask, bbox, pixel_values, criterion: str, mode: int,
              thresholds: Sequence[float], temperatures: Optional[Sequence[float]], want_all: bool,
-             blocking: bool = True, plan: Optional["ForwardPlan"] = None):
+             blocking: bool = True, plan: Optional["ForwardPlan"] = None, images=None):
         """One forward through the engine; `plan` given: a run of that captured forward plan instead (same inputs,
-        same outputs)."""
-        if pixel_values is None:
-            raise ValueError("pixel_values are required (multimodal and image-only paths)")
+        same outputs).  `images` (uint8 pages, see `mmee.images`) in place of `pixel_values`: with host inputs and no
+        plan the forward is `mmee_forward_images`; otherwise the pages are preprocessed on the device first
+        (`preprocess_images`) and the forward runs on the device (results read back for host inputs)."""
+        if images is not None:
+            if pixel_values is not None:
+                raise ValueError("pass either pixel_values or images, not both")
+            images = as_packed(images)
+            n_docs, px_device = len(images), images.data.device
+        elif pixel_values is None:
+            raise ValueError("pixel_values (or images) are required (multimodal and image-only paths)")
+        else:
+            n_docs, px_device = pixel_values.shape[0], pixel_values.device
         if input_ids is None:
             if self.dims.n_text != 0:
                 raise ValueError("this engine was built for the multimodal path: input_ids and bbox are required "
                                  "(build it with ModelDims(n_text=0) for the image-only path)")
-            input_ids = torch.zeros((pixel_values.shape[0], 0), dtype=torch.int64, device=pixel_values.device)
+            input_ids = torch.zeros((n_docs, 0), dtype=torch.int64, device=px_device)
         B, T = input_ids.shape
         if T != self.dims.n_text:
             raise ValueError(f"expected {self.dims.n_text} text tokens (padding='max_length'), got {T}")
+        if images is not None and len(images) != B:
+            raise ValueError(f"{len(images)} images for {B} documents")
         if attention_mask is None:
             attention_mask = torch.ones_like(input_ids)
         if bbox is None:
             bbox = torch.zeros((B, T, 4), dtype=torch.long, device=input_ids.device)
         on_dev = input_ids.is_cuda
+        to_host = False
+        if images is not None and (on_dev or plan is not None):
+            pixel_values = self.preprocess_images(images)
+            images = None
+            if not on_dev:          # a plan over host inputs: run its device path and read the results back
+                input_ids, to_host, on_dev = input_ids.to(pixel_values.device), True, True
         dev = input_ids.device
         ids = input_ids.to(torch.int64).contiguous()
         msk = attention_mask.to(device=dev, dtype=torch.int64).contiguous()
         bb = bbox.to(device=dev, dtype=torch.int64).contiguous()
-        px = pixel_values.to(device=dev, dtype=torch.float32).contiguous()
+        px = None if images is not None else pixel_values.to(device=dev, dtype=torch.float32).contiguous()
         E1, K = self.n_exits + 1, self.dims.n_labels
         kw = dict(device=dev)
         logits = torch.empty((B, K), dtype=torch.float32, **kw)
@@ -238,6 +256,15 @@ class B200EEForSequenceClassification:
             if tmp.shape[0] != E1:
                 raise ValueError(f"temperatures must have {E1} entries (one per exit + final)")
             pol.temperatures = tmp.ctypes.data_as(C.POINTER(C.c_float))
+        if images is not None:      # host forward over uint8 pages
+            if images.data.is_cuda:
+                images = PackedImages(images.data.cpu(), images.offsets, images.sizes, images.channels)
+            img = images.c_struct()
+            _lib.check(self._lib.mmee_forward_images(self._h, B, C.c_void_p(ids.data_ptr()), C.c_void_p(bb.data_ptr()),
+                                                     C.c_void_p(msk.data_ptr()), C.byref(img), C.byref(pol),
+                                                     C.byref(out)))
+            return dict(logits=logits, exit_index=exit_index, criterion=crit, hist=hist, all_logits=all_l,
+                        all_head=all_h, all_crit=all_c, _keep=(ids, msk, bb, images, thr, tmp))
         args = (C.c_void_p(ids.data_ptr()), C.c_void_p(bb.data_ptr()), C.c_void_p(msk.data_ptr()),
                 C.c_void_p(px.data_ptr()), C.byref(pol), C.byref(out))
         if plan is None:
@@ -260,15 +287,20 @@ class B200EEForSequenceClassification:
                 _lib.check(self._lib.mmee_sync(self._h, C.c_void_p(stream)))
         else:
             _lib.check(fwd_host(*args))
-        return dict(logits=logits, exit_index=exit_index, criterion=crit, hist=hist, all_logits=all_l,
-                    all_head=all_h, all_crit=all_c, _keep=(ids, msk, bb, px, thr, tmp))
+        r = dict(logits=logits, exit_index=exit_index, criterion=crit, hist=hist, all_logits=all_l,
+                 all_head=all_h, all_crit=all_c, _keep=(ids, msk, bb, px, thr, tmp))
+        if to_host:
+            r.update({k: v.cpu() for k, v in r.items() if torch.is_tensor(v)})
+        return r
 
     # ------------------------------------------------------------------ reference-shaped forward (dense)
     def forward(self, input_ids=None, attention_mask=None, bbox=None, pixel_values=None, labels=None,
-                temperatures: Optional[Sequence[float]] = None, **unused) -> EESequenceClassifierOutput:
+                temperatures: Optional[Sequence[float]] = None, images=None, **unused) -> EESequenceClassifierOutput:
+        """`images`: uint8 pages (a `mmee.images.PackedImages` or what `pack_images` takes) instead of `pixel_values`;
+        the engine resizes and normalises them as the reference's image processor does.  Same for `infer*`."""
         crit_name = self.ee.inference_strategy
         r = self._run(input_ids, attention_mask, bbox, pixel_values, crit_name, 0,
-                      [float(self.ee.global_threshold)], temperatures, True)
+                      [float(self.ee.global_threshold)], temperatures, True, images=images)
         E, K = self.n_exits, self.dims.n_labels
         gate = self.ee.encoder_layer_strategy == "gate"
         n_head = 2 if gate else K
@@ -294,11 +326,11 @@ class B200EEForSequenceClassification:
     def infer(self, input_ids=None, attention_mask=None, bbox=None, pixel_values=None, labels=None,
               exit_threshold: Union[float, Sequence[float], None] = None,
               temperatures: Optional[Sequence[float]] = None, criterion: Optional[str] = None,
-              early_exit: bool = True, return_all: bool = False, **unused) -> EarlyExitResult:
+              early_exit: bool = True, return_all: bool = False, images=None, **unused) -> EarlyExitResult:
         thr = self.ee.global_threshold if exit_threshold is None else exit_threshold
         crit_name = criterion or self._default_criterion()
         r = self._run(input_ids, attention_mask, bbox, pixel_values, crit_name, 1 if early_exit else 0,
-                      np.atleast_1d(np.asarray(thr, dtype=np.float32)), temperatures, return_all)
+                      np.atleast_1d(np.asarray(thr, dtype=np.float32)), temperatures, return_all, images=images)
         return self._early_exit_result(r, return_all)
 
     def _early_exit_result(self, r, return_all: bool) -> EarlyExitResult:
@@ -317,19 +349,37 @@ class B200EEForSequenceClassification:
     def infer_device(self, input_ids=None, attention_mask=None, bbox=None, pixel_values=None, labels=None,
                      exit_threshold: Union[float, Sequence[float], None] = None,
                      temperatures: Optional[Sequence[float]] = None, criterion: Optional[str] = None,
-                     early_exit: bool = True, **unused) -> Dict[str, torch.Tensor]:
+                     early_exit: bool = True, images=None, **unused) -> Dict[str, torch.Tensor]:
         """`infer` without the device->host read-back: results stay on the GPU (logits f32 [B,K], exit_index i32 [B],
         criterion f32 [B], hist i64 [E+1]) and the call is asynchronous on the current stream — what the
         data-parallel gather (`mmee.dist`) and pipelined callers want.  Inputs must be CUDA tensors."""
         thr = self.ee.global_threshold if exit_threshold is None else exit_threshold
         crit_name = criterion or self._default_criterion()
         r = self._run(input_ids, attention_mask, bbox, pixel_values, crit_name, 1 if early_exit else 0,
-                      np.atleast_1d(np.asarray(thr, dtype=np.float32)), temperatures, False, blocking=False)
+                      np.atleast_1d(np.asarray(thr, dtype=np.float32)), temperatures, False, blocking=False,
+                      images=images)
         return self._device_result(r)
 
     @staticmethod
     def _device_result(r) -> Dict[str, torch.Tensor]:
         return {"logits": r["logits"], "exit_index": r["exit_index"], "criterion": r["criterion"], "hist": r["hist"]}
+
+    # ------------------------------------------------------------------ uint8 images
+    def preprocess_images(self, images) -> torch.Tensor:
+        """Pixel values f32 [B, 3, S, S] (S = dims.image) on this engine's GPU from uint8 pages (a `PackedImages` or
+        what `mmee.images.pack_images` takes), computed on the device and asynchronous on the current stream:
+        Pillow's bilinear resize to S x S, then (r / 255 - 0.5) / 0.5, bit for bit as the reference's LayoutLMv3 image
+        processor (`mmee_preprocess_images`)."""
+        p = as_packed(images)
+        dev = torch.device("cuda", self.device_index)
+        data = p.data.to(dev, non_blocking=True)
+        S = self.dims.image
+        out = torch.empty((len(p), 3, S, S), dtype=torch.float32, device=dev)
+        img = p.c_struct(data)
+        stream = torch.cuda.current_stream(dev).cuda_stream or 1     # see _run: 0 would mean "engine stream, sync"
+        _lib.check(self._lib.mmee_preprocess_images(self._h, len(p), C.byref(img), C.c_void_p(out.data_ptr()),
+                                                    C.c_void_p(stream)))
+        return out
 
     # ------------------------------------------------------------------ captured forwards
     def plan(self, batch_size: int, criterion: Optional[str] = None, early_exit: bool = True,
@@ -351,6 +401,8 @@ class B200EEForSequenceClassification:
         """Enqueue one early-exit forward over HOST tensors (pinned memory recommended) and return a ticket without
         waiting; at most two tickets may be outstanding.  The upload of this batch overlaps the forward of the
         previous one (`mmee_forward_submit`).  Pass the ticket to `infer_collect`."""
+        if "images" in unused:
+            raise ValueError("infer_submit takes pixel_values only (use infer / infer_device for uint8 images)")
         if pixel_values is None or pixel_values.is_cuda:
             raise ValueError("infer_submit takes host tensors (use infer / infer_device for CUDA tensors)")
         if input_ids is None:
@@ -473,7 +525,7 @@ class ForwardPlan:
         mode = 1 if (self.early_exit if early_exit is None else early_exit) else 0
         return m._run(batch.get("input_ids"), batch.get("attention_mask"), batch.get("bbox"),
                       batch.get("pixel_values"), crit_name, mode, np.atleast_1d(np.asarray(thr, dtype=np.float32)),
-                      temperatures, want_all, blocking=blocking, plan=self)
+                      temperatures, want_all, blocking=blocking, plan=self, images=batch.get("images"))
 
     def infer(self, exit_threshold: Union[float, Sequence[float], None] = None,
               temperatures: Optional[Sequence[float]] = None, criterion: Optional[str] = None,
