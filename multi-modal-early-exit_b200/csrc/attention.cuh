@@ -30,6 +30,7 @@
 #include <type_traits>
 
 #include "ptx.cuh"
+#include "tmap.h"
 
 namespace mmee {
 
@@ -741,6 +742,55 @@ attention_kernel(const __grid_constant__ AttMaps maps, const AttArgs args) {
     tc_fence_after();
     tmem_dealloc<SMEM::TMEM_COLS>(tmem_base);
   }
+}
+
+// ------------------------------------------------------------------ host side: tensor maps, launch
+// The engine and the attention tests (tests/kernels/attention_harness.cu) both launch through these, so the tests run
+// the engine's own launch.
+
+// The maps of the layouts above over m_rows rows of qk and `docs` documents (V^T by slot, the bias by document).
+// split (fp32 engine mode): the *_lo pointers are the low parts; otherwise they are ignored and lo = hi.
+inline AttMaps attention_maps(const void* qk, const void* qk_lo, const void* vt, const void* vt_lo, const void* bias,
+                              const void* bias_lo, uint64_t m_rows, int H, int heads, int seq, int docs, int kv_pitch,
+                              int bias_pitch, bool split) {
+  const uint64_t vt_rows = static_cast<uint64_t>(docs) * heads * 64, bias_rows = static_cast<uint64_t>(docs) * heads * seq;
+  auto make = [&](const void* q, const void* v, const void* b, CUtensorMap& mq, CUtensorMap& mk, CUtensorMap& mv,
+                  CUtensorMap& mb) {
+    mq = make_tmap_2d_sw128(q, m_rows, 2 * H, 2 * H, ATT_BQ);
+    mk = make_tmap_2d_sw128(q, m_rows, 2 * H, 2 * H, ATT_BKV);
+    mv = make_tmap_2d_sw128(v, vt_rows, kv_pitch, kv_pitch, 64);
+    mb = make_tmap_2d_sw128(b, bias_rows, bias_pitch, bias_pitch, ATT_BQ, CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
+  };
+  AttMaps m;
+  make(qk, vt, bias, m.q, m.k, m.vt, m.bias);
+  if (split) make(qk_lo, vt_lo, bias_lo, m.q_lo, m.k_lo, m.vt_lo, m.bias_lo);
+  else { m.q_lo = m.q; m.k_lo = m.k; m.vt_lo = m.vt; m.bias_lo = m.bias; }
+  return m;
+}
+
+// One attention launch on `device` (an ordinal, passed in so a launch queries nothing) with `sms` SMs: ATT_CTAS_PER_SM
+// CTAs per SM, or one for split (the fp32-mode kernel) and for one_cta (bf16: 16 KB of extra dynamic shared memory
+// keep a second CTA off the SM).  trace (bf16): the kTrace instantiation.  Static (internal linkage): every library
+// built from this header (the engine, a test harness) keeps its own attribute cache for its own copy of the kernels.
+static inline void launch_attention(int device, int sms, const AttMaps& maps, const AttArgs& args, bool split, bool trace,
+                                    bool one_cta, cudaStream_t st) {
+  // the shared-memory attribute is per device; it is set by the first launch, before a plan captures a forward
+  static bool configured[64] = {};
+  if (!configured[device & 63]) {
+    CUDA_OK(cudaFuncSetAttribute(attention_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmem::DYN_BYTES + 16 * 1024));
+    CUDA_OK(cudaFuncSetAttribute(attention_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmem::DYN_BYTES + 16 * 1024));
+    CUDA_OK(cudaFuncSetAttribute(attention_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmemT<true>::DYN_BYTES));
+    configured[device & 63] = true;
+  }
+  const int grid = sms * ((split || one_cta) ? 1 : ATT_CTAS_PER_SM);
+  const size_t smem = AttSmem::DYN_BYTES + (one_cta ? 16 * 1024 : 0);
+  if (split)
+    attention_kernel<false, true><<<grid, ATT_THREADS, AttSmemT<true>::DYN_BYTES, st>>>(maps, args);
+  else if (trace)
+    attention_kernel<true, false><<<grid, ATT_THREADS, smem, st>>>(maps, args);
+  else
+    attention_kernel<false, false><<<grid, ATT_THREADS, smem, st>>>(maps, args);
+  CUDA_OK(cudaGetLastError());
 }
 
 }  // namespace mmee

@@ -33,13 +33,6 @@ namespace {
 
 thread_local std::string g_err;
 
-#define CUDA_OK(x)                                                                                   \
-  do {                                                                                               \
-    cudaError_t e_ = (x);                                                                            \
-    if (e_ != cudaSuccess)                                                                           \
-      throw std::runtime_error(std::string(#x) + ": " + cudaGetErrorString(e_) + " @" + std::to_string(__LINE__)); \
-  } while (0)
-
 template <typename T>
 struct DevBuf {
   T* p = nullptr;
@@ -86,19 +79,6 @@ __global__ void fill_nan_kernel(float* p, size_t n) {
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   if (i < n) p[i] = __int_as_float(0x7fc00000);
 }
-// dst[new slot] = src[slot_src[new slot]] for whole documents of `doc_bytes` bytes (a multiple of 16); used only after
-// an embedding-level exit.
-__global__ void gather_slots_kernel(const void* __restrict__ src, void* __restrict__ dst,
-                                    const int* __restrict__ slot_src, const int* __restrict__ n_dev, size_t doc_bytes) {
-  const int slot = blockIdx.y;
-  if (slot >= *n_dev) return;
-  const size_t per_doc = doc_bytes / 16;
-  const uint4* s = reinterpret_cast<const uint4*>(src) + static_cast<size_t>(slot_src[slot]) * per_doc;
-  uint4* d = reinterpret_cast<uint4*>(dst) + static_cast<size_t>(slot) * per_doc;
-  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < per_doc;
-       i += static_cast<size_t>(gridDim.x) * blockDim.x)
-    d[i] = s[i];
-}
 __global__ void hist_to_i64_kernel(const unsigned long long* h, long long* out, int n) {
   const int i = threadIdx.x;
   if (i < n) out[i] = static_cast<long long>(h[i]);
@@ -136,7 +116,6 @@ struct mmee_engine {
   int max_batch = 0;
   int H, L, heads, I, T, P, S, K, n_vis, n_patch, kdim_patch;
   int kv_pitch = 768, bias_pitch = 768;
-  int bias_width = 768;
   bool split = false;              // fp32 engine mode (mmee_model_desc.compute_dtype == MMEE_DTYPE_FP32): split-bf16 operands
   // ragged encoder layout (norm_exit.cuh): kept tokens per document and the row plans of two consecutive exit stages
   DevBuf<int> doc_len, kept_idx, plan_row0[2], plan_qt_slot[2], plan_n_qt[2];
@@ -187,10 +166,8 @@ struct mmee_engine {
   DevBuf<__nv_bfloat16> QKlo, VTlo, CTXlo, MIDlo, PATCHlo;   // fp32 engine mode: low parts of every other GEMM / attention operand
   DevBuf<__half> BIASlo;                    // fp32 engine mode: low part of the attention bias
   DevBuf<float> X32[2], A132;               // fp32 engine mode: the residual stream itself in fp32 (exact residual adds)
-  // fp32 engine mode: the tensor core adds each K = 16 product block into the fp32 accumulator with truncation, so the
-  // error of a long contraction grows linearly with K (measured: 2e-5 relative at K = 3072 x 3 segments).  The MLP-down
-  // GEMM (K = inter) therefore runs in chunks of <= 1024: every chunk is its own launch whose residual epilogue adds
-  // the running sum Y in fp32 (round to nearest).
+  // fp32 engine mode: the MLP-down GEMM runs in K chunks (gemm_kchunk; measured without them: 2e-5 relative error at
+  // K = 3072 x 3 segments); every chunk after the first adds to the running sum Y
   int kchunk = 0, n_kchunks = 1;
   std::vector<CUtensorMap> t_mid_c, t_mid_lo_c;
   DevBuf<float> zero_bias;
@@ -205,8 +182,9 @@ struct mmee_engine {
   bool trace_on = false;
   int n_kv_tiles = 6;
   DevBuf<int> posid;
-  CUtensorMap t_x[2], t_qk, t_k64, t_vt, t_bias, t_ctx, t_a1, t_mid, t_patch;
-  CUtensorMap t_x_lo[2], t_qk_lo, t_k64_lo, t_vt_lo, t_bias_lo, t_ctx_lo, t_a1_lo, t_mid_lo, t_patch_lo;   // fp32 engine mode
+  CUtensorMap t_x[2], t_ctx, t_a1, t_mid, t_patch;
+  CUtensorMap t_x_lo[2], t_ctx_lo, t_a1_lo, t_mid_lo, t_patch_lo;   // fp32 engine mode
+  AttMaps att_maps;
 
   // bookkeeping (device)
   DevBuf<int> n_dev, m_dev;                 // [stages]
@@ -346,56 +324,13 @@ void load_head(mmee_engine* e, HeadW& h, const std::string& prefix, int n_out) {
   upload_f32(h.out_b, need(e, prefix + ".out_proj.bias", {n_out}));
 }
 
-template <int BN, int EPI, bool SPLIT>
-void launch_gemm_t(mmee_engine* e, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ta_lo,
-                   const CUtensorMap& tb_lo, const GemmArgs& a, cudaStream_t st) {
-  auto kern = gemm_tc_kernel<BN, EPI, SPLIT>;
-  static bool configured_dev[64] = {};
-  bool& configured = configured_dev[e->device & 63];   // the attribute is per device
-  if (!configured) {
-    CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmSmem<BN>::DYN_BYTES));
-    configured = true;
-  }
-  kern<<<e->sms, GEMM_THREADS, GemmSmem<BN>::DYN_BYTES, st>>>(ta, tb, ta_lo, tb_lo, a);
-  CUDA_OK(cudaGetLastError());
-  e->launches++;
-}
-
-// BLOCK_N = 256 shapes run on the CTA-pair (cta_group::2) kernel; its weight tensor maps use 128-row boxes
-// (each CTA of the pair stages half of the 256 output columns), see wbox().
-template <int EPI, bool SPLIT>
-void launch_gemm_pair(mmee_engine* e, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ta_lo,
-                      const CUtensorMap& tb_lo, const GemmArgs& a, cudaStream_t st) {
-  auto kern = gemm_tc_pair_kernel<EPI, SPLIT>;
-  using PS = GemmPairSmemT<gemm_pair_epi_warps<EPI>()>;
-  static bool configured_dev[64] = {};
-  bool& configured = configured_dev[e->device & 63];   // the attribute is per device
-  if (!configured) {
-    CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, PS::DYN_BYTES));
-    configured = true;
-  }
-  kern<<<e->sms & ~1, PS::THREADS, PS::DYN_BYTES, st>>>(ta, tb, ta_lo, tb_lo, a);
-  CUDA_OK(cudaGetLastError());
-  e->launches++;
-}
-
-// ta_lo / tb_lo: tensor maps of the operands' low parts; both given = fp32 engine mode (three k segments)
+// ta_lo / tb_lo: tensor maps of the operands' low parts (fp32 engine mode: three k segments); unused in bf16 mode
 template <int EPI>
-void launch_gemm(mmee_engine* e, int bn, const CUtensorMap& ta, const CUtensorMap& tb, const GemmArgs& a,
-                 cudaStream_t st, const CUtensorMap* ta_lo = nullptr, const CUtensorMap* tb_lo = nullptr) {
-  if (e->split) {
-    if (!ta_lo || !tb_lo) throw std::runtime_error("fp32 mode: GEMM launched without the low-part tensor maps");
-    if (bn == 256) launch_gemm_pair<EPI, true>(e, ta, tb, *ta_lo, *tb_lo, a, st);
-    else launch_gemm_t<128, EPI, true>(e, ta, tb, *ta_lo, *tb_lo, a, st);
-  } else {
-    if (bn == 256) launch_gemm_pair<EPI, false>(e, ta, tb, ta, tb, a, st);
-    else launch_gemm_t<128, EPI, false>(e, ta, tb, ta, tb, a, st);
-  }
+void run_gemm(mmee_engine* e, int bn, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ta_lo,
+              const CUtensorMap& tb_lo, const GemmArgs& a, cudaStream_t st) {
+  launch_gemm<EPI>(e->device, e->sms, bn, e->split, ta, tb, ta_lo, tb_lo, a, st);
+  e->launches++;
 }
-
-int wbox(int bn) { return bn == 256 ? 128 : bn; }   // weight TMA box rows for a GEMM family with BLOCK_N = bn
-
-int pick_bn(int n) { return (n % 256 == 0) ? 256 : 128; }
 
 template <typename F>
 void launch_nv(int H, F&& f) {   // dispatch on values-per-lane for the warp-per-row kernels
@@ -548,23 +483,23 @@ void finalize(mmee_engine* e) {
     upload_f32(w.bo2, need(e, lp + "output.dense.bias", {H}));
     upload_f32(w.ln2_w, need(e, lp + "output.LayerNorm.weight", {H}));
     upload_f32(w.ln2_b, need(e, lp + "output.LayerNorm.bias", {H}));
-    w.t_wqkv = make_tmap_2d_sw128(w.wqkv.p, 3 * H, H, H, wbox(e->bn_qkv));
-    w.t_wo = make_tmap_2d_sw128(w.wo.p, H, H, H, wbox(e->bn_h));
-    w.t_wi = make_tmap_2d_sw128(w.wi.p, I, H, H, wbox(e->bn_i));
-    w.t_wo2 = make_tmap_2d_sw128(w.wo2.p, H, I, I, wbox(e->bn_h));
+    w.t_wqkv = gemm_w_map(w.wqkv.p, 3 * H, H, H, e->bn_qkv);
+    w.t_wo = gemm_w_map(w.wo.p, H, H, H, e->bn_h);
+    w.t_wi = gemm_w_map(w.wi.p, I, H, H, e->bn_i);
+    w.t_wo2 = gemm_w_map(w.wo2.p, H, I, I, e->bn_h);
     if (split) {
-      w.t_wqkv_lo = make_tmap_2d_sw128(w.wqkv_lo.p, 3 * H, H, H, wbox(e->bn_qkv));
-      w.t_wo_lo = make_tmap_2d_sw128(w.wo_lo.p, H, H, H, wbox(e->bn_h));
-      w.t_wi_lo = make_tmap_2d_sw128(w.wi_lo.p, I, H, H, wbox(e->bn_i));
-      w.t_wo2_lo = make_tmap_2d_sw128(w.wo2_lo.p, H, I, I, wbox(e->bn_h));
+      w.t_wqkv_lo = gemm_w_map(w.wqkv_lo.p, 3 * H, H, H, e->bn_qkv);
+      w.t_wo_lo = gemm_w_map(w.wo_lo.p, H, H, H, e->bn_h);
+      w.t_wi_lo = gemm_w_map(w.wi_lo.p, I, H, H, e->bn_i);
+      w.t_wo2_lo = gemm_w_map(w.wo2_lo.p, H, I, I, e->bn_h);
       for (int c = 0; c < e->n_kchunks; ++c) {
-        w.t_wo2_c.push_back(make_tmap_2d_sw128(w.wo2.p + static_cast<size_t>(c) * e->kchunk, H, e->kchunk, I, wbox(e->bn_h)));
-        w.t_wo2_lo_c.push_back(make_tmap_2d_sw128(w.wo2_lo.p + static_cast<size_t>(c) * e->kchunk, H, e->kchunk, I, wbox(e->bn_h)));
+        w.t_wo2_c.push_back(gemm_w_map(w.wo2.p, H, e->kchunk, I, e->bn_h, static_cast<size_t>(c) * e->kchunk));
+        w.t_wo2_lo_c.push_back(gemm_w_map(w.wo2_lo.p, H, e->kchunk, I, e->bn_h, static_cast<size_t>(c) * e->kchunk));
       }
     }
   }
-  e->t_patch_w = make_tmap_2d_sw128(e->patch_w.p, H, e->kdim_patch, e->kdim_patch, wbox(e->bn_h));
-  if (split) e->t_patch_w_lo = make_tmap_2d_sw128(e->patch_w_lo.p, H, e->kdim_patch, e->kdim_patch, wbox(e->bn_h));
+  e->t_patch_w = gemm_w_map(e->patch_w.p, H, e->kdim_patch, e->kdim_patch, e->bn_h);
+  if (split) e->t_patch_w_lo = gemm_w_map(e->patch_w_lo.p, H, e->kdim_patch, e->kdim_patch, e->bn_h);
 
   const int n_head_out = d.head_kind == 0 ? d.n_labels : 2;
   e->exit_heads.resize(d.n_exits);
@@ -656,13 +591,10 @@ void allocate(mmee_engine* e) {
   if (e->split) e->BIASlo.alloc(static_cast<size_t>(B) * heads * S * e->bias_pitch + 64 * 1024, true);
   e->posid.alloc(static_cast<size_t>(B) * e->T);
 
-  e->t_x[0] = make_tmap_2d_sw128(e->X[0].p, M, H, H, 128);
-  e->t_x[1] = make_tmap_2d_sw128(e->X[1].p, M, H, H, 128);
-  e->t_qk = make_tmap_2d_sw128(e->QK.p, M, 2 * H, 2 * H, 128);
-  e->t_vt = make_tmap_2d_sw128(e->VT.p, static_cast<uint64_t>(B) * heads * 64, e->kv_pitch, e->kv_pitch, 64);
-  e->t_k64 = make_tmap_2d_sw128(e->QK.p, M, 2 * H, 2 * H, ATT_BKV);
-  e->t_bias = make_tmap_2d_sw128(e->BIAS.p, static_cast<uint64_t>(B) * heads * S, e->bias_width, e->bias_pitch, ATT_BQ,
-                                 CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
+  e->t_x[0] = gemm_a_map(e->X[0].p, M, H, H);
+  e->t_x[1] = gemm_a_map(e->X[1].p, M, H, H);
+  e->att_maps = attention_maps(e->QK.p, e->QKlo.p, e->VT.p, e->VTlo.p, e->BIAS.p, e->BIASlo.p, M, H, heads, S, B,
+                               e->kv_pitch, e->bias_pitch, e->split);
   e->n_kv_tiles = (S + ATT_BKV - 1) / ATT_BKV;
   if (e->n_kv_tiles > ATT_MAX_KV_TILES) throw std::runtime_error("too many key tiles");
   e->maskadd.alloc(static_cast<size_t>(B) * e->kv_pitch, true);
@@ -677,27 +609,22 @@ void allocate(mmee_engine* e) {
     e->plan_n_qt[i].alloc(1, true);
   }
   e->att_trace.alloc(4096, true);
-  e->t_ctx = make_tmap_2d_sw128(e->CTX.p, M, H, H, 128);
-  e->t_a1 = make_tmap_2d_sw128(e->A1.p, M, H, H, 128);
-  e->t_mid = make_tmap_2d_sw128(e->MID.p, M, I, I, 128);
-  e->t_patch = make_tmap_2d_sw128(e->PATCH.p, mp, e->kdim_patch, e->kdim_patch, 128);
+  e->t_ctx = gemm_a_map(e->CTX.p, M, H, H);
+  e->t_a1 = gemm_a_map(e->A1.p, M, H, H);
+  e->t_mid = gemm_a_map(e->MID.p, M, I, I);
+  e->t_patch = gemm_a_map(e->PATCH.p, mp, e->kdim_patch, e->kdim_patch);
   if (e->split) {
-    e->t_x_lo[0] = make_tmap_2d_sw128(e->Xlo[0].p, M, H, H, 128);
-    e->t_x_lo[1] = make_tmap_2d_sw128(e->Xlo[1].p, M, H, H, 128);
-    e->t_qk_lo = make_tmap_2d_sw128(e->QKlo.p, M, 2 * H, 2 * H, 128);
-    e->t_k64_lo = make_tmap_2d_sw128(e->QKlo.p, M, 2 * H, 2 * H, ATT_BKV);
-    e->t_vt_lo = make_tmap_2d_sw128(e->VTlo.p, static_cast<uint64_t>(B) * heads * 64, e->kv_pitch, e->kv_pitch, 64);
-    e->t_bias_lo = make_tmap_2d_sw128(e->BIASlo.p, static_cast<uint64_t>(B) * heads * S, e->bias_width, e->bias_pitch, ATT_BQ,
-                                      CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
-    e->t_ctx_lo = make_tmap_2d_sw128(e->CTXlo.p, M, H, H, 128);
-    e->t_a1_lo = make_tmap_2d_sw128(e->A1lo.p, M, H, H, 128);
-    e->t_mid_lo = make_tmap_2d_sw128(e->MIDlo.p, M, I, I, 128);
-    e->t_patch_lo = make_tmap_2d_sw128(e->PATCHlo.p, mp, e->kdim_patch, e->kdim_patch, 128);
-    e->kchunk = (I > 1024 && I % 1024 == 0) ? 1024 : ((I > 768 && I % 768 == 0) ? 768 : I);
+    e->t_x_lo[0] = gemm_a_map(e->Xlo[0].p, M, H, H);
+    e->t_x_lo[1] = gemm_a_map(e->Xlo[1].p, M, H, H);
+    e->t_ctx_lo = gemm_a_map(e->CTXlo.p, M, H, H);
+    e->t_a1_lo = gemm_a_map(e->A1lo.p, M, H, H);
+    e->t_mid_lo = gemm_a_map(e->MIDlo.p, M, I, I);
+    e->t_patch_lo = gemm_a_map(e->PATCHlo.p, mp, e->kdim_patch, e->kdim_patch);
+    e->kchunk = gemm_kchunk(I);
     e->n_kchunks = I / e->kchunk;
     for (int c = 0; c < e->n_kchunks; ++c) {
-      e->t_mid_c.push_back(make_tmap_2d_sw128(e->MID.p + static_cast<size_t>(c) * e->kchunk, M, e->kchunk, I, 128));
-      e->t_mid_lo_c.push_back(make_tmap_2d_sw128(e->MIDlo.p + static_cast<size_t>(c) * e->kchunk, M, e->kchunk, I, 128));
+      e->t_mid_c.push_back(gemm_a_map(e->MID.p, M, e->kchunk, I, static_cast<size_t>(c) * e->kchunk));
+      e->t_mid_lo_c.push_back(gemm_a_map(e->MIDlo.p, M, e->kchunk, I, static_cast<size_t>(c) * e->kchunk));
     }
     e->zero_bias.alloc(H, true);
   }
@@ -987,7 +914,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     GemmArgs ga{};
     ga.m_dev = nullptr; ga.m_static = B * e->n_patch; ga.N = H; ga.K = e->kdim_patch; ga.bias = e->patch_b.p;
     ga.out = e->VIS.p; ga.ld_out = H; ga.pos = e->pos_embed.p; ga.n_patch = e->n_patch; ga.n_vis = e->n_vis;
-    launch_gemm<EPI_PATCH>(e, e->bn_h, e->t_patch, e->t_patch_w, ga, st, &e->t_patch_lo, &e->t_patch_w_lo);
+    run_gemm<EPI_PATCH>(e, e->bn_h, e->t_patch, e->t_patch_w, e->t_patch_lo, e->t_patch_w_lo, ga, st);
     const int blocks = std::min((B * e->n_vis + 7) / 8, e->sms * 16);
     const int wp = keep_normed ? 1 : 0;
     switch (H % 128 == 0 ? H / 128 : 0) {
@@ -1083,7 +1010,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
   // over ALL 709 tokens, pads included, as the reference does) works on dense [slot, 709] rows; from here on a document
   // owns only the rows of its kept tokens.  The same pass moves the survivors of the concat exit to their new slots.
   {
-    plan_rows_kernel<<<1, 256, 0, st>>>(e->slot_doc[sd].p, e->doc_len.p, e->n_dev.p + stage, plan_view(e, rp), e->m_dev.p + stage, ATT_BQ);
+    launch_plan_rows(e->slot_doc[sd].p, e->doc_len.p, e->n_dev.p + stage, plan_view(e, rp), e->m_dev.p + stage, ATT_BQ, st);
     // where the dense rows of slot s live: by document (no vision / text exit: the embedding stage ran in document
     // order), else by the slot numbering of the embedding stage (identity, or new -> old after the concat exit left)
     const int* src_index = !modality_exits ? e->slot_doc[sd].p : ((any_embedding_exit && leave) ? e->slot_src.p : nullptr);
@@ -1116,7 +1043,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     ga.m_dev = mdev; ga.N = 3 * H; ga.K = H; ga.bias = w.bqkv.p; ga.out = e->QK.p; ga.out_lo = e->QKlo.p; ga.ld_out = 2 * H;
     ga.vt = e->VT.p; ga.vt_lo = e->VTlo.p; ga.qk_cols = 2 * H; ga.row0 = e->plan_row0[rp].p; ga.n_slots_dev = e->n_dev.p + stage;
     ga.kv_pitch = e->kv_pitch; ga.heads = heads;
-    launch_gemm<EPI_QKV>(e, e->bn_qkv, e->t_x[cur], w.t_wqkv, ga, st, &e->t_x_lo[cur], &w.t_wqkv_lo);
+    run_gemm<EPI_QKV>(e, e->bn_qkv, e->t_x[cur], w.t_wqkv, e->t_x_lo[cur], w.t_wqkv_lo, ga, st);
     mark(e, "gemm", st);
 
     AttArgs aa;
@@ -1124,33 +1051,11 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
     aa.ctx = e->CTX.p; aa.ctx_lo = e->CTXlo.p; aa.H = H; aa.heads = heads; aa.seq = S;
     aa.tail16 = (e->tail16 && !split) ? 1 : 0;
     aa.experiment = getenv("MMEE_ATT_EXPERIMENT") ? atoi(getenv("MMEE_ATT_EXPERIMENT")) : 0; aa.err_flag = e->err_flags.p; aa.trace = e->att_trace.p;
-    {
-      static bool configured_dev[64] = {};
-      bool& configured = configured_dev[e->device & 63];   // the attribute is per device
-      if (!configured) {
-        CUDA_OK(cudaFuncSetAttribute(attention_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmem::DYN_BYTES + 16 * 1024));
-        CUDA_OK(cudaFuncSetAttribute(attention_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmem::DYN_BYTES + 16 * 1024));
-        CUDA_OK(cudaFuncSetAttribute(attention_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmemT<true>::DYN_BYTES));
-        configured = true;
-      }
-      AttMaps am;
-      am.q = e->t_qk; am.k = e->t_k64; am.vt = e->t_vt; am.bias = e->t_bias;
-      if (split) { am.q_lo = e->t_qk_lo; am.k_lo = e->t_k64_lo; am.vt_lo = e->t_vt_lo; am.bias_lo = e->t_bias_lo; }
-      else { am.q_lo = e->t_qk; am.k_lo = e->t_k64; am.vt_lo = e->t_vt; am.bias_lo = e->t_bias; }
-      // developer experiment MMEE_ATT_ONE_CTA=1: one attention CTA per SM (extra dynamic shared memory keeps the second
-      // one out) — shows what a softmax warp does when it has its scheduler's MUFU to itself
-      static const bool one_cta = getenv("MMEE_ATT_ONE_CTA") != nullptr;
-      const int att_grid = e->sms * ((split || one_cta) ? 1 : ATT_CTAS_PER_SM);
-      const size_t att_smem = AttSmem::DYN_BYTES + (one_cta ? 16 * 1024 : 0);
-      if (split)
-        attention_kernel<false, true><<<att_grid, ATT_THREADS, AttSmemT<true>::DYN_BYTES, st>>>(am, aa);
-      else if (e->trace_on && l == 0)
-        attention_kernel<true, false><<<att_grid, ATT_THREADS, att_smem, st>>>(am, aa);
-      else
-        attention_kernel<false, false><<<att_grid, ATT_THREADS, att_smem, st>>>(am, aa);
-      CUDA_OK(cudaGetLastError());
-      e->launches++;
-    }
+    // developer experiment MMEE_ATT_ONE_CTA=1: one attention CTA per SM (extra dynamic shared memory keeps the second
+    // one out) — shows what a softmax warp does when it has its scheduler's MUFU to itself
+    static const bool one_cta = getenv("MMEE_ATT_ONE_CTA") != nullptr;
+    launch_attention(e->device, e->sms, e->att_maps, aa, split, e->trace_on && l == 0, one_cta, st);
+    e->launches++;
     mark(e, "attention", st);
 
     // y_resid: the out-projection writes Y2 (Y still holds the previous layer's MLP-down sums, from which this residual
@@ -1169,7 +1074,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
       ga.resid_y = e->Y.p; ga.resid_stats = e->ln_stats2.p; ga.resid_src = e->ln_src2.p;
       ga.resid_w = pw.ln2_w.p; ga.resid_b = pw.ln2_b.p;
     }
-    launch_gemm<EPI_RESID_F32>(e, e->bn_h, e->t_ctx, w.t_wo, ga, st, &e->t_ctx_lo, &w.t_wo_lo);
+    run_gemm<EPI_RESID_F32>(e, e->bn_h, e->t_ctx, w.t_wo, e->t_ctx_lo, w.t_wo_lo, ga, st);
     mark(e, "gemm", st);
     launch_ln(e, y_att, e->A1.p, yr ? nullptr : e->A1lo.p, split ? e->A132.p : nullptr, w.ln1_w.p, w.ln1_b.p, B, mdev, nullptr,
               plan_view(e, rp), plan_view(e, rp), e->n_dev.p + stage, st, yr ? e->ln_stats1.p : nullptr, nullptr);
@@ -1178,7 +1083,7 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
 
     ga = GemmArgs{};
     ga.m_dev = mdev; ga.N = I; ga.K = H; ga.bias = w.bi.p; ga.out = e->MID.p; ga.out_lo = e->MIDlo.p; ga.ld_out = I;
-    launch_gemm<EPI_GELU_BF16>(e, e->bn_i, e->t_a1, w.t_wi, ga, st, &e->t_a1_lo, &w.t_wi_lo);
+    run_gemm<EPI_GELU_BF16>(e, e->bn_i, e->t_a1, w.t_wi, e->t_a1_lo, w.t_wi_lo, ga, st);
     ga = GemmArgs{};
     ga.m_dev = mdev; ga.N = H; ga.K = I; ga.bias = w.bo2.p; ga.out = e->Y.p; ga.ld_out = H; ga.resid = e->A1.p;
     ga.resid_lo = yr ? nullptr : e->A1lo.p;
@@ -1193,10 +1098,10 @@ void forward_device(mmee_engine* e, int B, const int64_t* ids, const int64_t* bb
       for (int c = 0; c < e->n_kchunks; ++c) {
         ga.K = e->kchunk;
         if (c > 0) { ga.bias = e->zero_bias.p; ga.resid_f32 = e->Y.p; }
-        launch_gemm<EPI_RESID_F32>(e, e->bn_h, e->t_mid_c[c], w.t_wo2_c[c], ga, st, &e->t_mid_lo_c[c], &w.t_wo2_lo_c[c]);
+        run_gemm<EPI_RESID_F32>(e, e->bn_h, e->t_mid_c[c], w.t_wo2_c[c], e->t_mid_lo_c[c], w.t_wo2_lo_c[c], ga, st);
       }
     } else {
-      launch_gemm<EPI_RESID_F32>(e, e->bn_h, e->t_mid, w.t_wo2, ga, st, &e->t_mid_lo, &w.t_wo2_lo);
+      run_gemm<EPI_RESID_F32>(e, e->bn_h, e->t_mid, w.t_wo2, e->t_mid_lo, w.t_wo2_lo, ga, st);
     }
     mark(e, "gemm", st);
 
@@ -1622,15 +1527,13 @@ int mmee_create(const mmee_model_desc* desc, int device, int max_batch, mmee_eng
   // a last key tile with <= 16 real keys (an unpadded document, S = 709: 5) runs as a 16-key tile (N = 16 MMAs, a quarter of
   // the softmax work); decided per document by the attention kernel (documents are ragged)
   e->tail16 = !getenv("MMEE_NO_TAIL16");
-  e->bias_width = e->bias_pitch;
   if (e->kv_pitch > 1024) throw std::runtime_error("sequence too long for keymask_kernel");
   e->sms = prop.multiProcessorCount;
   if (const char* pr = getenv("MMEE_PRECISE_RESIDUAL")) e->precise_residual = pr[0] != '0';   // developer A/B switch
   if (e->split) e->precise_residual = true;   // fp32 engine mode: split operands everywhere (and full 64-key tiles in attention)
   e->y_resid = e->precise_residual && !e->split && e->H % 128 == 0;
   if (const char* yr = getenv("MMEE_Y_RESID")) e->y_resid = e->y_resid && yr[0] != '0';   // developer A/B switch
-  e->bn_h = pick_bn(e->H); e->bn_qkv = pick_bn(e->H) ; e->bn_i = pick_bn(e->I);
-  if ((2 * e->H) % e->bn_qkv) e->bn_qkv = 128;
+  e->bn_h = gemm_block_n(e->H); e->bn_qkv = gemm_block_n_qkv(e->H); e->bn_i = gemm_block_n(e->I);
   try {
     CUDA_OK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     CUDA_OK(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));

@@ -21,6 +21,7 @@
 #include <cuda.h>
 
 #include "ptx.cuh"
+#include "tmap.h"
 
 namespace mmee {
 
@@ -644,6 +645,75 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     tc_fence_after();
     tmem_dealloc_pair<512>(tmem_base);
   }
+}
+
+// ------------------------------------------------------------------ host side: shapes, tensor maps, launch
+// The engine and the GEMM tests (tests/kernels/gemm_harness.cu) both launch through these, so the tests run the
+// engine's own launch.
+
+// BLOCK_N of a GEMM with N = n output columns: 256 (the CTA-pair kernel) when it divides n, else 128.
+inline int gemm_block_n(int n) { return (n % 256 == 0) ? 256 : 128; }
+
+// BLOCK_N of the QKV GEMM (N = 3H): a tile holds either Q|K or V^T columns, so 2H must be a multiple of it.
+inline int gemm_block_n_qkv(int H) {
+  const int bn = gemm_block_n(H);
+  return (2 * H) % bn ? 128 : bn;
+}
+
+// fp32 engine mode: the tensor core adds each K = 16 product block into the fp32 accumulator with truncation, so the
+// error of a long contraction grows linearly with K.  The MLP-down GEMM (K = I) therefore runs in K chunks of this many
+// columns, each its own launch whose residual epilogue adds the running sum in fp32 (round to nearest).
+inline int gemm_kchunk(int I) { return (I > 1024 && I % 1024 == 0) ? 1024 : ((I > 768 && I % 768 == 0) ? 768 : I); }
+
+// Weight TMA box rows: each CTA of a pair (BLOCK_N = 256) stages half of the 256 output columns.
+inline int gemm_wbox(int bn) { return bn == 256 ? 128 : bn; }
+
+// A operand: columns [col0, col0 + K) of `rows` bf16 rows at row pitch `pitch` (col0 > 0: a K chunk).
+inline CUtensorMap gemm_a_map(const __nv_bfloat16* a, uint64_t rows, uint64_t K, uint64_t pitch, size_t col0 = 0) {
+  return make_tmap_2d_sw128(a + col0, rows, K, pitch, GEMM_BLOCK_M);
+}
+
+// Weight [N, K] of a GEMM family with BLOCK_N = bn: columns [col0, col0 + K) of bf16 rows at row pitch `pitch`.
+inline CUtensorMap gemm_w_map(const __nv_bfloat16* w, uint64_t N, uint64_t K, uint64_t pitch, int bn, size_t col0 = 0) {
+  return make_tmap_2d_sw128(w + col0, N, K, pitch, gemm_wbox(bn));
+}
+
+// static (internal linkage) here and below: every library built from this header (the engine, a test harness) keeps its
+// own attribute cache for its own copy of the kernels.  A static of an inline function would be one object per process.
+template <int EPI, bool SPLIT>
+static void launch_gemm_kernel(int device, int sms, int bn, const CUtensorMap& ta, const CUtensorMap& tb,
+                               const CUtensorMap& ta_lo, const CUtensorMap& tb_lo, const GemmArgs& a, cudaStream_t st,
+                               int grid) {
+  // the shared-memory attribute is per device; it is set by the first launch, before a plan captures a forward
+  if (bn == 256) {
+    using PS = GemmPairSmemT<gemm_pair_epi_warps<EPI>()>;
+    static bool configured[64] = {};
+    if (!configured[device & 63]) {
+      CUDA_OK(cudaFuncSetAttribute(gemm_tc_pair_kernel<EPI, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   PS::DYN_BYTES));
+      configured[device & 63] = true;
+    }
+    gemm_tc_pair_kernel<EPI, SPLIT><<<grid ? grid : (sms & ~1), PS::THREADS, PS::DYN_BYTES, st>>>(ta, tb, ta_lo, tb_lo, a);
+  } else {
+    static bool configured[64] = {};
+    if (!configured[device & 63]) {
+      CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<128, EPI, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   GemmSmem<128>::DYN_BYTES));
+      configured[device & 63] = true;
+    }
+    gemm_tc_kernel<128, EPI, SPLIT><<<grid ? grid : sms, GEMM_THREADS, GemmSmem<128>::DYN_BYTES, st>>>(ta, tb, ta_lo, tb_lo, a);
+  }
+  CUDA_OK(cudaGetLastError());
+}
+
+// One GEMM on `device` (an ordinal, passed in so a launch queries nothing) with `sms` SMs.  bn: 128 (gemm_tc_kernel)
+// or 256 (gemm_tc_pair_kernel, CTA pairs).  split (fp32 engine mode): ta_lo / tb_lo are the low parts' maps; in bf16
+// mode they are ignored.  grid 0: one CTA per SM (pairs: an even count); another grid gives the same result.
+template <int EPI>
+static void launch_gemm(int device, int sms, int bn, bool split, const CUtensorMap& ta, const CUtensorMap& tb,
+                        const CUtensorMap& ta_lo, const CUtensorMap& tb_lo, const GemmArgs& a, cudaStream_t st, int grid = 0) {
+  if (split) launch_gemm_kernel<EPI, true>(device, sms, bn, ta, tb, ta_lo, tb_lo, a, st, grid);
+  else launch_gemm_kernel<EPI, false>(device, sms, bn, ta, tb, ta, tb, a, st, grid);
 }
 
 }  // namespace mmee

@@ -95,6 +95,10 @@ __global__ void __launch_bounds__(256) plan_rows_kernel(const int* __restrict__ 
   __shared__ int s_scan[72];
   plan_rows_block(slot_doc, doc_len, *n_active_dev, out, m_dev, q_rows, s_scan);
 }
+inline void launch_plan_rows(const int* slot_doc, const int* doc_len, const int* n_active_dev, const SlotRows& out,
+                             int* m_dev, int q_rows, cudaStream_t st) {
+  plan_rows_kernel<<<1, 256, 0, st>>>(slot_doc, doc_len, n_active_dev, out, m_dev, q_rows);
+}
 
 // dense embedding output -> ragged encoder input: dst[row0[s] + r] = src[src_index[s] * seq + token(r)], token(r) = the
 // r-th kept text token of the slot's document, then the visual tokens.  `elem_bytes` per element (2: bf16 rows, 4: fp32

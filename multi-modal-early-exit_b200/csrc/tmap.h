@@ -8,6 +8,14 @@
 #include <stdexcept>
 #include <string>
 
+// Host code: a failing CUDA runtime call throws, naming the call and the line.
+#define CUDA_OK(x)                                                                                   \
+  do {                                                                                               \
+    cudaError_t e_ = (x);                                                                            \
+    if (e_ != cudaSuccess)                                                                           \
+      throw std::runtime_error(std::string(#x) + ": " + cudaGetErrorString(e_) + " @" + std::to_string(__LINE__)); \
+  } while (0)
+
 namespace mmee {
 
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,

@@ -2,10 +2,8 @@
 // csrc/norm_exit.cuh) on caller-built inputs, for tests/test_attention_gpu.py.  Test-only code: the engine never links
 // it.  All pointers are device pointers (torch tensors); both calls synchronise and return a cudaError_t (0 = success).
 //
-// The tensor maps, the shared-memory attribute, the grid and the launch are literal copies of the engine's lines
-// (engine.cu, allocate(): t_qk / t_k64 / t_vt / t_bias; forward_device(): the attention launch of an encoder layer),
-// so the kernel sees exactly the operands it sees inside a forward.  When the attention kernel or its launch changes,
-// this file changes with it.
+// Argument marshalling only: the tensor maps (attention_maps) and the launches (launch_attention, launch_plan_rows)
+// are the engine's own, from the host-side sections of attention.cuh and norm_exit.cuh.
 #include <cuda.h>
 #include <cuda_runtime.h>
 
@@ -19,17 +17,9 @@
 
 using namespace mmee;
 
-#define CUDA_OK(x)                                                                                   \
-  do {                                                                                               \
-    cudaError_t e_ = (x);                                                                            \
-    if (e_ != cudaSuccess)                                                                           \
-      throw std::runtime_error(std::string(#x) + ": " + cudaGetErrorString(e_) + " @" + std::to_string(__LINE__)); \
-  } while (0)
-
 extern "C" {
 
-// engine.cu forward_device(): plan_rows_kernel<<<1, 256, 0, st>>>(slot_doc, doc_len, n_dev + stage, plan_view(e, rp),
-// m_dev + stage, ATT_BQ).  n_dev: device int, the number of slots.
+// The row plan of the encoder's first stage.  n_dev: device int, the number of slots.
 int att_plan(const int* slot_doc, const int* doc_len, const int* n_dev, int* row0, int* meta, int* qt_slot, int* n_qt,
              int* m_dev) {
   SlotRows r;
@@ -37,7 +27,7 @@ int att_plan(const int* slot_doc, const int* doc_len, const int* n_dev, int* row
   r.meta = reinterpret_cast<int4*>(meta);
   r.qt_slot = qt_slot;
   r.n_qt_dev = n_qt;
-  plan_rows_kernel<<<1, 256>>>(slot_doc, doc_len, n_dev, r, m_dev, ATT_BQ);
+  launch_plan_rows(slot_doc, doc_len, n_dev, r, m_dev, ATT_BQ, 0);
   cudaError_t err = cudaGetLastError();
   if (err == cudaSuccess) err = cudaDeviceSynchronize();
   return static_cast<int>(err);
@@ -55,43 +45,16 @@ int att_run(const void* qk, const void* qk_lo, const void* vt, const void* vt_lo
             int H, int heads, int seq, int n_docs, int kv_pitch, int bias_pitch, int tail16, int split, int one_cta) {
   try {
     int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int B = n_docs, S = seq, bias_width = bias_pitch;
-    const uint64_t M = static_cast<uint64_t>(m_rows);
-    // engine.cu allocate()
-    const CUtensorMap t_qk = make_tmap_2d_sw128(qk, M, 2 * H, 2 * H, 128);
-    const CUtensorMap t_vt = make_tmap_2d_sw128(vt, static_cast<uint64_t>(B) * heads * 64, kv_pitch, kv_pitch, 64);
-    const CUtensorMap t_k64 = make_tmap_2d_sw128(qk, M, 2 * H, 2 * H, ATT_BKV);
-    const CUtensorMap t_bias = make_tmap_2d_sw128(bias, static_cast<uint64_t>(B) * heads * S, bias_width, bias_pitch, ATT_BQ,
-                                                  CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
-    CUtensorMap t_qk_lo = t_qk, t_k64_lo = t_k64, t_vt_lo = t_vt, t_bias_lo = t_bias;
-    if (split) {
-      t_qk_lo = make_tmap_2d_sw128(qk_lo, M, 2 * H, 2 * H, 128);
-      t_k64_lo = make_tmap_2d_sw128(qk_lo, M, 2 * H, 2 * H, ATT_BKV);
-      t_vt_lo = make_tmap_2d_sw128(vt_lo, static_cast<uint64_t>(B) * heads * 64, kv_pitch, kv_pitch, 64);
-      t_bias_lo = make_tmap_2d_sw128(bias_lo, static_cast<uint64_t>(B) * heads * S, bias_width, bias_pitch, ATT_BQ,
-                                     CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
-    }
-    // engine.cu forward_device(), attention of an encoder layer
+    CUDA_OK(cudaGetDevice(&dev));
+    CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const AttMaps am = attention_maps(qk, qk_lo, vt, vt_lo, bias, bias_lo, static_cast<uint64_t>(m_rows), H, heads, seq,
+                                      n_docs, kv_pitch, bias_pitch, split);
     AttArgs aa{};
     aa.slot_meta = reinterpret_cast<const int4*>(meta); aa.qt_slot = qt_slot; aa.n_qt_dev = n_qt;
-    aa.ctx = static_cast<__nv_bfloat16*>(ctx); aa.ctx_lo = static_cast<__nv_bfloat16*>(ctx_lo); aa.H = H; aa.heads = heads; aa.seq = S;
+    aa.ctx = static_cast<__nv_bfloat16*>(ctx); aa.ctx_lo = static_cast<__nv_bfloat16*>(ctx_lo); aa.H = H; aa.heads = heads; aa.seq = seq;
     aa.tail16 = (tail16 && !split) ? 1 : 0;
     aa.experiment = 0; aa.err_flag = err_flag; aa.trace = nullptr;
-    CUDA_OK(cudaFuncSetAttribute(attention_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmem::DYN_BYTES + 16 * 1024));
-    CUDA_OK(cudaFuncSetAttribute(attention_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttSmemT<true>::DYN_BYTES));
-    AttMaps am;
-    am.q = t_qk; am.k = t_k64; am.vt = t_vt; am.bias = t_bias;
-    if (split) { am.q_lo = t_qk_lo; am.k_lo = t_k64_lo; am.vt_lo = t_vt_lo; am.bias_lo = t_bias_lo; }
-    else { am.q_lo = t_qk; am.k_lo = t_k64; am.vt_lo = t_vt; am.bias_lo = t_bias; }
-    const int att_grid = sms * ((split || one_cta) ? 1 : ATT_CTAS_PER_SM);
-    const size_t att_smem = AttSmem::DYN_BYTES + (one_cta ? 16 * 1024 : 0);
-    if (split)
-      attention_kernel<false, true><<<att_grid, ATT_THREADS, AttSmemT<true>::DYN_BYTES>>>(am, aa);
-    else
-      attention_kernel<false, false><<<att_grid, ATT_THREADS, att_smem>>>(am, aa);
-    CUDA_OK(cudaGetLastError());
+    launch_attention(dev, sms, am, aa, split, false, one_cta, 0);
     CUDA_OK(cudaDeviceSynchronize());
     return 0;
   } catch (const std::exception& ex) {

@@ -55,7 +55,14 @@ def gemm(tmp_path_factory):
     lib.gemm_run.argtypes = ([i] * 4 + [p, p, q, q, p, p, q, p, i, i, i, p, p, p, i] + [p] * 8 +
                              [i, p, p, i, p, p, i, i, p, i, i])
     lib.gemm_run.restype = i
+    for rule in (lib.gemm_bn, lib.gemm_bn_qkv, lib.gemm_k_chunk):
+        rule.argtypes, rule.restype = [i], i
+    global _lib
+    _lib = lib
     return lib
+
+
+_lib = None   # the harness the gemm fixture loaded: its exports are the engine's shape rules (gemm.cuh)
 
 
 def _p(t):
@@ -63,19 +70,18 @@ def _p(t):
 
 
 def pick_bn(n):
-    """engine.cu pick_bn: BLOCK_N of a GEMM family with N = n columns."""
-    return 256 if n % 256 == 0 else 128
+    """gemm_block_n: BLOCK_N of a GEMM family with N = n columns."""
+    return _lib.gemm_bn(n)
 
 
 def bn_qkv(H):
-    """engine.cu mmee_create: the QKV GEMM's BLOCK_N."""
-    bn = pick_bn(H)
-    return 128 if (2 * H) % bn else bn
+    """gemm_block_n_qkv: the QKV GEMM's BLOCK_N."""
+    return _lib.gemm_bn_qkv(H)
 
 
 def kchunk(I):
-    """engine.cu allocate(): K chunk of the fp32-mode MLP-down."""
-    return 1024 if (I > 1024 and I % 1024 == 0) else (768 if (I > 768 and I % 768 == 0) else I)
+    """gemm_kchunk: K chunk of the fp32-mode MLP-down."""
+    return _lib.gemm_k_chunk(I)
 
 
 def split_bf16(x):
